@@ -2,7 +2,7 @@
 """Headline benchmark: frames/sec through the four trackers (BASELINE.json metric) on synthetic frames.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|eager] [--config all4|players|pose|court|ball]
-                  [--batch B] [--res 1080p|4k|720p] [--strong [--frames N]]
+                  [--batch B] [--res 1080p|4k|720p] [--strong [--frames N]] [--dump-outputs DIR]
 
 One *step* = one batch of `--batch` frames through the hot path of the selected trackers (default all four:
 PlayerTracker YOLOv8n-detect, PlayerKeypointsTracker YOLOv8n-pose 13x3 @1280, KeypointsTracker YOLOv8n-pose 12x3 @640,
@@ -321,12 +321,50 @@ def make_ckpts(which, rank, world, dev):
         # sparse heads: a handful of players per frame like a real padel rally (the dense defaults are for parity tests)
         mk = {"detect": lambda: OW.make_yolo("detect", cls_mean=-5.0), "pose13": lambda: OW.make_yolo("pose13", cls_mean=-5.7),
               "court12": lambda: OW.make_yolo("court12"), "tracknet": OW.make_tracknet}
-        ckpts = {KIND[k]: mk[KIND[k]]() for k in which}
+        # the heads are standardised with CPU convolutions whose last bits depend on the thread count: one thread makes
+        # the weights, and so every output, the same on any host
+        threads = torch.get_num_threads()
+        torch.set_num_threads(1)
+        try:
+            ckpts = {KIND[k]: mk[KIND[k]]() for k in which}
+        finally:
+            torch.set_num_threads(threads)
     if world > 1:
         box = [ckpts]
         dist.broadcast_object_list(box, src=0, device=dev)
         ckpts = box[0]
     return ckpts
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out, path: Path):
+    """What a caller of the fused pass receives for one batch, as float64 tables with one row per object, written to
+    path/<tracker>.npy.  `frame` is the index within the batch (ball: the tracker's frame number).
+      players: frame, x1, y1, x2, y2, confidence, class_id, tracker id (-1: none)
+      pose:    frame, then x, y of the 13 keypoints of one player
+      court:   frame, then x, y of the 12 keypoints ordered by id
+      ball:    frame, x, y, visibility
+    Tables above DUMP_BYTES together keep the same seeded sample of rows on every run."""
+    rows = {
+        "players": [[f, *p.xyxy, p.confidence, p.class_id, -1 if p.id is None else p.id]
+                    for f, ps in enumerate(out.get("players", [])) for p in ps],
+        "pose": [[f, *(v for k in pk.player_keypoints for v in k.xy)]
+                 for f, pks in enumerate(out.get("pose", [])) for pk in pks],
+        "court": [[f, *(v for k in kps.keypoints for v in k.xy)] for f, kps in enumerate(out.get("court", [])) if len(kps)],
+        "ball": [[f, *xyv] for f, xyv in out.get("ball", {}).items()],
+    }
+    width = {"players": 8, "pose": 27, "court": 25, "ball": 4}
+    tables = {k: np.array(v, dtype=np.float64).reshape(-1, width[k]) for k, v in rows.items() if k in out}
+    total = sum(t.nbytes for t in tables.values())
+    if total > DUMP_BYTES:
+        rng = np.random.default_rng(0)
+        tables = {k: t[np.sort(rng.choice(len(t), len(t) * DUMP_BYTES // total, replace=False))]
+                  for k, t in tables.items()}
+    path.mkdir(parents=True, exist_ok=True)
+    for k, t in tables.items():
+        np.save(path / f"{k}.npy", t)
 
 
 def run_strong(args, rank, world, local, dev):
@@ -379,7 +417,7 @@ def run_strong(args, rank, world, local, dev):
     if rank == 0:
         sampler.start()
     walls, tms, launches, nobj = [], [], 0, 0
-    for _ in range(max(1, args.steps)):
+    for _ in range(args.steps):
         w_, tm, launches, nobj = one_pass()
         walls.append(w_)
         tms.append(tm)
@@ -421,7 +459,13 @@ def main():
     ap.add_argument("--frames", type=int, default=4096, help="--strong: frames of the fixed job")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-host", action="store_true", help="cProfile the timed region's host side (stderr)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the tracker outputs of the last timed step as DIR/<tracker>.npy (float64 tables)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.strong):
+        ap.error("--dump-outputs covers the default fused pass only (--impl ours, no --strong)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -480,10 +524,10 @@ def main():
         ball._pipe.push_frames(dev_batches[0][:7])  # prime the 8-frame window so every step yields B windows
 
     def run_steps(batches, steps):
-        nd = 0
+        nd, out = 0, None
         for out in fused.run(batches[i % NBUF] for i in range(steps)):
             nd += sum(len(p) for k in ("players", "pose") if k in out for p in out[k])
-        return nd
+        return nd, out
 
     import gc
 
@@ -499,7 +543,7 @@ def main():
         e0.record()
         if os.environ.get("PADEL_B200_NCU") == "1":  # `ncu --profile-from-start off`: capture the timed region only
             torch.cuda.profiler.start()
-        nd = run_steps(batches, steps)
+        nd, out = run_steps(batches, steps)
         if os.environ.get("PADEL_B200_NCU") == "1":
             torch.cuda.synchronize()
             torch.cuda.profiler.stop()
@@ -512,7 +556,7 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dist.barrier()
             ms, wall = t[0].item(), t[1].item() / 1e3
-        return ms, wall, L.lib().pb_launch_count() - l0, nd
+        return ms, wall, L.lib().pb_launch_count() - l0, nd, out
 
     run_steps(dev_batches, args.warmup)
     sampler = ClockSampler(local)
@@ -524,12 +568,14 @@ def main():
 
         pr = cProfile.Profile()
         pr.enable()
-    ms_dev, wall_dev, launches, ndet = timed(dev_batches, args.steps)
+    ms_dev, wall_dev, launches, ndet, last = timed(dev_batches, args.steps)
     if args.profile_host:
         pr.disable()
         pstats.Stats(pr, stream=sys.stderr).sort_stats("cumulative").print_stats(35)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, Path(args.dump_outputs))
     run_steps(host_batches, 2)
-    ms_e2e, wall_e2e, _, _ = timed(host_batches, args.steps)
+    ms_e2e, wall_e2e, _, _, _ = timed(host_batches, args.steps)
     clocks = sampler.stop() if rank == 0 else None
 
     frames_total = B * args.steps * world

@@ -14,7 +14,8 @@ yolo_glue_ref.npz — the reference's OWN PlayerKeypointsTracker.predict_sample 
                 rally.mp4 crops under tests/golden/rally/: what the reference's glue (processor, predict arguments,
                 ratio scaling, id mapping, object construction) makes of a given model output.  ultralytics itself
                 stays unpinned (absent); for PlayerTracker the `supervision` names are bound to this repo's sv_compat
-                (supervision is absent too), so only the reference's own lines are pinned there.
+                (supervision is absent too), so only the reference's own lines are pinned there.  The oracle YOLO
+                results the glue was given are stored with it (oracle_*).
 """
 import sys
 import tempfile
@@ -145,11 +146,29 @@ def yolo_glue_golden():
     import trackers.keypoints_tracker.keypoints_tracker as rkt
     import trackers.players_keypoints_tracker.players_keypoints_tracker as rpk
     import trackers.players_tracker.players_tracker as rpt
+    from oracle import yolov8 as OY
     from padel_analytics_b200.trackers import sv_compat
 
     frames = rally_frames()
     H, W = frames[0].shape[:2]
     out = {"H": H, "W": W, "n": len(frames)}
+    # the oracle YOLO results the reference glue consumed (oracle_<tracker>_{boxes,kpts}_<frame>): the test feeds them
+    # to the product glue, whose exact comparison must not depend on how the host's CPU convolutions round
+    calls = []
+    predict = OY.YOLO.predict
+
+    def spy(self, *a, **k):
+        res = predict(self, *a, **k)
+        calls.append([(r.boxes.data.numpy().copy(), None if r.keypoints is None else r.keypoints.data.numpy().copy())
+                      for r in res])
+        return res
+
+    def keep(name, i, res):
+        out[f"oracle_{name}_boxes_{i}"], kp = res
+        if kp is not None:
+            out[f"oracle_{name}_kpts_{i}"] = kp
+
+    OY.YOLO.predict = spy
     with tempfile.TemporaryDirectory() as td:
         paths = {}
         for kind in ("detect", "pose13", "court12"):
@@ -162,6 +181,7 @@ def yolo_glue_golden():
             arr = np.array([[kp.xy for kp in player.player_keypoints] for player in p.players_keypoints], dtype=np.float64)
             assert arr.shape[0] >= 3 and arr.shape[1:] == (13, 2), arr.shape
             out[f"pose_{i}"] = arr
+            keep("pose", i, calls[-1][i])
         out["pose_names"] = np.array([kp.name for kp in preds[0].players_keypoints[0].player_keypoints])
         # --- KeypointsTracker: exactly one detection per frame (q5) -> per-frame CONF via a subclass attribute
         net = OW.load_yolo(glue_ckpt("court12"))
@@ -172,6 +192,7 @@ def yolo_glue_golden():
             cls = type("CourtOne", (rkt.KeypointsTracker,), {"CONF": conf})
             kt = cls(paths["court12"], batch_size=1, model_type="yolo")
             (kp,) = kt.predict_sample([f])
+            keep("court", i, calls[-1][0])
             ks = sorted(kp.keypoints, key=lambda k: k.id)
             assert [k.id for k in ks] == list(range(12))
             out[f"court_{i}"] = np.array([k.xy for k in ks], dtype=np.float64)
@@ -187,8 +208,10 @@ def yolo_glue_golden():
             for i, p in enumerate(preds):
                 out[f"players_{i}"] = np.array([[*pl.xyxy, pl.confidence, pl.class_id, -1 if pl.id is None else pl.id]
                                                 for pl in p.players], dtype=np.float64).reshape(-1, 7)
+                keep("players", i, calls[-1][i])
         finally:
             rpt.sv = sys.modules["supervision"]
+            OY.YOLO.predict = predict
     # --- KeypointsTracker(model_type="resnet") (keypoints_tracker.py:158-167,276-312): torchvision's resnet50 is
     # installed, only the `pretrained=True` download must be avoided (the state dict is loaded over it anyway)
     import torchvision

@@ -23,7 +23,9 @@ def test_tracknet_forward_matches_reference_golden():
     x = torch.rand((1, 27, 32, 64), generator=torch.Generator().manual_seed(int(g["seed"])))
     with torch.no_grad():
         y = net(x)
-    assert np.array_equal(y.numpy(), g["y"])  # same torch ops in the same order: bit-identical
+    # same torch ops in the same order, but the seeded weights and the forward run on CPU convolutions whose last bits
+    # depend on the host's thread count (up to ~6e-6 here); bit-identical only on a host like the golden's
+    assert np.abs(y.numpy() - g["y"]).max() < 5e-5
 
 
 def test_ball_stage_matches_reference_golden():
@@ -130,7 +132,10 @@ def test_tracker_glue_reproduces_reference_golden():
     """tests/golden/yolo_glue_ref.npz was produced by the UNMODIFIED reference tracker classes (predict_sample of
     PlayerKeypointsTracker / KeypointsTracker / PlayerTracker) driving the oracle YOLO on the committed rally.mp4 crops.
     The product trackers' host glue (processor semantics, predict arguments, ratio scaling, id mapping, result objects)
-    fed with the same oracle results must reproduce it EXACTLY; the GPU tests then only have to show engine == oracle."""
+    fed with the same oracle results must reproduce it EXACTLY; the GPU tests then only have to show engine == oracle.
+    The golden also stores the oracle results the reference glue was given.  The glue is fed those, because the seeded
+    checkpoints and the oracle run on CPU convolutions whose last bits depend on the host's thread count; the oracle
+    recomputed here must match them to that rounding."""
     import cv2
     from PIL import Image
 
@@ -148,11 +153,31 @@ def test_tracker_glue_reproduces_reference_golden():
     rgb = [cv2.cvtColor(f, cv2.COLOR_BGR2RGB) for f in frames]
     pil = [Image.fromarray(f).resize((640, 640)) for f in rgb]
 
+    def stored(kind, i, like):
+        """The stored oracle result of frame i, as the Result `like` (the recomputed one) is laid out."""
+        kp = f"oracle_{kind}_kpts_{i}"
+        return OY.Result(OY.Boxes(torch.from_numpy(g[f"oracle_{kind}_boxes_{i}"])),
+                         OY.Keypoints(torch.from_numpy(g[kp])) if kp in g.files else None, like.names, like.orig_shape)
+
+    def same_detections(res, ref):
+        """Same detections; box edges to 0.1 px (the seeded heads' multi-modal DFL edges are ill-conditioned, see
+        tests/parity.py: last-bit changes of the weights move them by up to ~0.01 px), scores and keypoints to 1e-3."""
+        assert len(res) == len(ref)
+        for r, s in zip(res, ref):
+            assert r.boxes.data.shape == s.boxes.data.shape
+            assert torch.allclose(r.boxes.xyxy, s.boxes.xyxy, rtol=0, atol=0.1)
+            assert torch.allclose(r.boxes.data[:, 4:], s.boxes.data[:, 4:], rtol=0, atol=1e-3)
+            assert (r.keypoints is None) == (s.keypoints is None)
+            if s.keypoints is not None:
+                assert torch.allclose(r.keypoints.data, s.keypoints.data, rtol=0, atol=1e-3)
+
     # pose (players_keypoints_tracker.py:271-322)
     pk = object.__new__(PlayerKeypointsTracker)  # no CUDA here: skip the engine, keep the class constants
     pk.train_image_size = 640
     res = OY.YOLO(OW.load_yolo(glue_ckpt("pose13"))).predict(pil, conf=pk.CONF, iou=pk.IOU, imgsz=640, classes=[0])
-    out = pk.postprocess(res, (H, W))
+    ref = [stored("pose", i, r) for i, r in enumerate(res)]
+    same_detections(res, ref)
+    out = pk.postprocess(ref, (H, W))
     assert list(g["pose_names"]) == PlayerKeypoints.KEYPOINTS_NAMES
     for i, p in enumerate(out):
         arr = np.array([[kp.xy for kp in pl.player_keypoints] for pl in p.players_keypoints], dtype=np.float64)
@@ -163,10 +188,12 @@ def test_tracker_glue_reproduces_reference_golden():
     net = OW.load_yolo(glue_ckpt("court12"))
     kt = object.__new__(KeypointsTracker)
     for i, f in enumerate(frames):
-        conf = court_conf_for_single_detection(net, f)
-        assert conf == float(g["court_conf"][i])
+        conf = float(g["court_conf"][i])
+        assert abs(court_conf_for_single_detection(net, f) - conf) < 1e-5
         res = OY.YOLO(net).predict([pil[i]], conf=conf, iou=kt.IOU, imgsz=kt.TRAIN_IMAGE_SIZE, max_det=kt.NUMBER_KEYPOINTS)
-        (kp,) = kt.postprocess(res, (H, W))
+        ref = [stored("court", i, res[0])]
+        same_detections(res, ref)
+        (kp,) = kt.postprocess(ref, (H, W))
         assert [k.id for k in kp.keypoints] == list(range(12))
         assert np.array_equal(np.array([k.xy for k in kp.keypoints]), g[f"court_{i}"]), f"court frame {i}"
 
@@ -175,7 +202,9 @@ def test_tracker_glue_reproduces_reference_golden():
     pt.polygon_zone = sv.PolygonZone(np.array([[0, 0], [W, 0], [W, H], [0, H]]), frame_resolution_wh=(W, H))
     pt.video_info_post_init(sv.VideoInfo(width=W, height=H, fps=25.0, total_frames=len(frames)))
     res = OY.YOLO(OW.load_yolo(glue_ckpt("detect"))).predict(rgb, conf=pt.CONF, iou=pt.IOU, imgsz=pt.IMGSZ, classes=[0])
-    for i, p in enumerate(pt.postprocess(res)):
+    ref = [stored("players", i, r) for i, r in enumerate(res)]
+    same_detections(res, ref)
+    for i, p in enumerate(pt.postprocess(ref)):
         arr = np.array([[*pl.xyxy, pl.confidence, pl.class_id, -1 if pl.id is None else pl.id] for pl in p.players],
                        dtype=np.float64).reshape(-1, 7)
         assert np.array_equal(arr, g[f"players_{i}"]), f"players frame {i}"
