@@ -49,11 +49,6 @@ extern "C" {
 
 const char* pb_last_error(void);
 
-/* Options captured by the conv plans built AFTER this call (pb_program_add_conv, pb_conv2d): sm_limit > 0 sizes their
- * persistent grids for that many SMs instead of the whole device (a program meant to run beside other streams leaves
- * the remaining SMs to them); pdl = 1 / 0 turns programmatic dependent launch between consecutive kernels on / off for
- * those plans, -1 = the process default (on, PADEL_B200_PDL=0 disables).  (0, -1) restores the defaults. */
-void pb_set_plan_options(int sm_limit, int pdl);
 int pb_version(void);
 /* Number of kernels this library has launched since load (bench.py's gpu_launches). */
 long long pb_launch_count(void);
@@ -90,7 +85,8 @@ typedef struct pb_conv_desc {
    * pixels with a one-pixel zero border, i.e. a (N, H+2, W+2, 4) tensor whose pixel (y,x) sits at [y+1][x+1]
    * (written by pb_letterbox_u8_f16 / pb_u8_to_f16 with out_layout = 1).  Only for the 3x3 stride-2 stem conv:
    * C = 4, cin = 16, weight = half [3 filter rows][cout_pad][16] with k = s*4 + c (s = filter column, c = channel;
-   * k >= 12 and c == 3 are zero).  One TMA box of overlapping 16-element rows serves all three filter rows.  */
+   * k >= 12 and c == 3 are zero).  One dense TMA box of the tile's raw input pixels serves all three filter rows: the
+   * 16-element row of output pixel ow (padded pixels 2ow .. 2ow+3) is read in place, 16 bytes after its neighbour's. */
   int in_layout;
   /* 1: out = act(conv + bias + res) -- the torchvision ResNet Bottleneck (relu(bn3(conv3) + identity), the court
    * regressor of keypoints_tracker.py:158-167); 0: out = act(conv + bias) + res.                                 */
@@ -113,18 +109,11 @@ int pb_program_add_conv(pb_program* p, const pb_conv_desc* d);
 /* 2x2/s2 max-pool of a channel slice (TrackNet models.py:60,62,64) */
 int pb_program_add_maxpool2(pb_program* p, const void* in, int N, int H, int W, int C, int c_off, int c,
                             void* out, int out_C, int out_coff);
-/* nearest x2 upsample of a channel slice into a slice of a (2H,2W) tensor (models.py:66,68,70; YOLO layers 10,13) */
-int pb_program_add_upsample2(pb_program* p, const void* in, int N, int H, int W, int C, int c_off, int c,
-                             void* out, int out_C, int out_coff);
 /* SPPF pooling: slice0=[0,c) of buf is x'; writes maxpool5, maxpool5^2, maxpool5^3 into slices 1..3 */
 int pb_program_add_sppf_pool(pb_program* p, void* buf, int N, int H, int W, int C, int c);
-/* 1x1 conv (C -> n_out <= 8) + bias + sigmoid, half NHWC (N,H,W,C) -> float NCHW (N,n_out,H,W): the TrackNet predictor
- * (models.py:55,72-73). weight float [n_out][C], bias float [n_out]. */
-int pb_program_add_pointwise_head(pb_program* p, const void* in, int N, int H, int W, int C, const float* weight,
-                                  const float* bias, int n_out, float* out);
 int pb_program_num_ops(const pb_program* p);
 /* Kernel that op i launches: 0 conv_tc_kernel (per-tap boxes), 1 conv_halo_kernel (shared halo / stem), 2 maxpool2,
- * 3 upsample2, 4 sppf_pool, 5 pointwise_head; -1 if i is out of range. */
+ * 4 sppf_pool (3 and 5 were kernels of earlier versions); -1 if i is out of range. */
 int pb_program_op_kernel(const pb_program* p, int i);
 int pb_program_run(pb_program* p, void* stream);
 /* Run ops [first, last) only (per-layer timing / debugging). */

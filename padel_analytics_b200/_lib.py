@@ -56,9 +56,7 @@ SIGNATURES = {
     "pb_program_destroy": (None, [_p]),
     "pb_program_add_conv": (_i, [_p, C.POINTER(ConvDesc)]),
     "pb_program_add_maxpool2": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _p, _i, _i]),
-    "pb_program_add_upsample2": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _p, _i, _i]),
     "pb_program_add_sppf_pool": (_i, [_p, _p, _i, _i, _i, _i, _i]),
-    "pb_program_add_pointwise_head": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _i, _p]),
     "pb_program_num_ops": (_i, [_p]),
     "pb_program_op_kernel": (_i, [_p, _i]),
     "pb_program_run": (_i, [_p, _p]),
@@ -75,7 +73,6 @@ SIGNATURES = {
     "pb_resnet_stem7x7": (_i, [_p, _i, _i, _i, _p, _p, _p, _p]),
     "pb_maxpool3x3s2": (_i, [_p, _i, _i, _i, _i, _p, _p]),
     "pb_avgpool_fc_sigmoid": (_i, [_p, _i, _i, _i, _p, _p, _i, _p, _p]),
-    "pb_set_plan_options": (None, [_i, _i]),
     "pb_bytetrack_create": (_p, [C.c_double, _i, C.c_double, C.c_double]),
     "pb_bytetrack_destroy": (None, [_p]),
     "pb_bytetrack_reset": (None, [_p]),

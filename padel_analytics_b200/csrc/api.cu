@@ -21,15 +21,7 @@ void set_error(const char* fmt, ...) {
   g_error = buf;
 }
 
-static std::atomic<int> g_plan_sm_limit{0};
-static std::atomic<int> g_plan_pdl{-1};
-
-int plan_pdl() {
-  const int v = g_plan_pdl.load();
-  return v < 0 ? (pdl_enabled() ? 1 : 0) : (v != 0);
-}
-
-static int device_sms() {
+int num_sms() {
   static int sms = 0;
   static std::once_flag once;
   std::call_once(once, [] {
@@ -39,12 +31,6 @@ static int device_sms() {
       sms = 148;
   });
   return sms;
-}
-
-// SMs a plan may size its persistent grid for: all of them, or the budget set by pb_set_plan_options
-int num_sms() {
-  const int lim = g_plan_sm_limit.load(), sms = device_sms();
-  return (lim > 0 && lim < sms) ? lim : sms;
 }
 
 int ensure_dynamic_smem(const void* func, size_t bytes) {
@@ -63,26 +49,15 @@ int ensure_dynamic_smem(const void* func, size_t bytes) {
   return e;
 }
 
-bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("PADEL_B200_PDL");
-    on = (e && atoi(e) == 0) ? 0 : 1;
-  }
-  return on != 0;
-}
-
-enum class OpKind { Conv, MaxPool2, Upsample2, SppfPool, PointwiseHead };
+enum class OpKind { Conv, MaxPool2, SppfPool };
 
 struct Op {
   OpKind kind;
   std::unique_ptr<ConvPlan> conv;
-  // pool / upsample / sppf
+  // pool / sppf
   const void* in = nullptr;
   void* out = nullptr;
   int N = 0, H = 0, W = 0, C = 0, c_off = 0, c = 0, out_C = 0, out_coff = 0;
-  const float* hw = nullptr;  // pointwise head weights / bias
-  const float* hb = nullptr;
 };
 
 }  // namespace pb
@@ -97,11 +72,7 @@ extern "C" {
 
 const char* pb_last_error(void) { return g_error.c_str(); }
 
-void pb_set_plan_options(int sm_limit, int pdl) {
-  g_plan_sm_limit.store(sm_limit > 0 ? sm_limit : 0);
-  g_plan_pdl.store(pdl < 0 ? -1 : (pdl != 0));
-}
-int pb_version(void) { return 100; }
+int pb_version(void) { return 101; }
 long long pb_launch_count(void) { return g_launches.load(); }
 
 int pb_conv2d(const pb_conv_desc* d, void* stream) {
@@ -142,20 +113,8 @@ int pb_program_add_maxpool2(pb_program* p, const void* in, int N, int H, int W, 
                             int out_C, int out_coff) {
   return add_simple(p, OpKind::MaxPool2, in, N, H, W, C, c_off, c, out, out_C, out_coff);
 }
-int pb_program_add_upsample2(pb_program* p, const void* in, int N, int H, int W, int C, int c_off, int c, void* out,
-                             int out_C, int out_coff) {
-  return add_simple(p, OpKind::Upsample2, in, N, H, W, C, c_off, c, out, out_C, out_coff);
-}
 int pb_program_add_sppf_pool(pb_program* p, void* buf, int N, int H, int W, int C, int c) {
   return add_simple(p, OpKind::SppfPool, buf, N, H, W, C, 0, c, buf, C, 0);
-}
-
-int pb_program_add_pointwise_head(pb_program* p, const void* in, int N, int H, int W, int C, const float* weight,
-                                  const float* bias, int n_out, float* out) {
-  if (add_simple(p, OpKind::PointwiseHead, in, N, H, W, C, 0, n_out, out, 0, 0)) return 1;
-  p->ops.back().hw = weight;
-  p->ops.back().hb = bias;
-  return 0;
 }
 
 int pb_program_num_ops(const pb_program* p) { return p ? (int)p->ops.size() : 0; }
@@ -166,9 +125,7 @@ int pb_program_op_kernel(const pb_program* p, int i) {
   switch (op.kind) {
     case OpKind::Conv: return op.conv->variant == 1 ? 1 : 0;
     case OpKind::MaxPool2: return 2;
-    case OpKind::Upsample2: return 3;
     case OpKind::SppfPool: return 4;
-    case OpKind::PointwiseHead: return 5;
   }
   return -1;
 }
@@ -185,13 +142,7 @@ int pb_program_run_range(pb_program* p, int first, int last, void* stream) {
       case OpKind::MaxPool2:
         rc = launch_maxpool2(op.in, op.N, op.H, op.W, op.C, op.c_off, op.c, op.out, op.out_C, op.out_coff, s);
         break;
-      case OpKind::Upsample2:
-        rc = launch_upsample2(op.in, op.N, op.H, op.W, op.C, op.c_off, op.c, op.out, op.out_C, op.out_coff, s);
-        break;
       case OpKind::SppfPool: rc = launch_sppf_pool(op.out, op.N, op.H, op.W, op.C, op.c, s); break;
-      case OpKind::PointwiseHead:
-        rc = launch_pointwise_head(op.in, op.N, op.H, op.W, op.C, op.hw, op.hb, op.c, static_cast<float*>(op.out), s);
-        break;
     }
     if (rc) return rc;
   }

@@ -1,4 +1,4 @@
-// HBM-bound helper kernels on NHWC fp16 channel slices: 2x2 max-pool, nearest x2 upsample, SPPF pooling.
+// HBM-bound helper kernels on NHWC fp16 channel slices: 2x2 max-pool, SPPF pooling.
 // All move 16-byte vectors (8 channels) per thread with consecutive threads on consecutive channel groups,
 // so warps read/write contiguous NHWC runs.
 #include "internal.h"
@@ -36,25 +36,6 @@ __global__ void maxpool2_kernel(const __half* __restrict__ in, int N, int H, int
     const uint4 v11 = *reinterpret_cast<const uint4*>(b + (size_t)W * C + C);
     *reinterpret_cast<uint4*>(out + (((size_t)n * Ho + oh) * Wo + ow) * out_C + out_coff + g * 8) =
         hmax8(hmax8(v00, v01), hmax8(v10, v11));
-  }
-}
-
-// nn.Upsample(scale_factor=2) (nearest) — models.py:66,68,70 ; ultralytics layers 10/13 (SURVEY App. A.2)
-__global__ void upsample2_kernel(const __half* __restrict__ in, int N, int H, int W, int C, int c_off, int cg,
-                                 __half* __restrict__ out, int out_C, int out_coff) {
-  const int Ho = H * 2, Wo = W * 2;
-  const long total = (long)N * Ho * Wo * cg;
-  griddep_launch_dependents();
-  griddep_wait();
-  for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
-    const int g = (int)(i % cg);
-    long p = i / cg;
-    const int ow = (int)(p % Wo);
-    const int oh = (int)((p / Wo) % Ho);
-    const int n = (int)(p / ((long)Wo * Ho));
-    const uint4 v =
-        *reinterpret_cast<const uint4*>(in + (((size_t)n * H + oh / 2) * W + ow / 2) * C + c_off + g * 8);
-    *reinterpret_cast<uint4*>(out + (((size_t)n * Ho + oh) * Wo + ow) * out_C + out_coff + g * 8) = v;
   }
 }
 
@@ -101,70 +82,6 @@ __global__ void __launch_bounds__(256) sppf_pool_kernel(__half* __restrict__ buf
   }
 }
 
-// TrackNet predictor: 1x1 conv (C -> n_out <= 8) + bias + sigmoid, fp16 NHWC in, fp32 NCHW planes out
-// (/root/reference/trackers/ball_tracker/models.py:55,72-73).  HBM-bound (C*2 bytes in, n_out*4 bytes out per pixel):
-// a block stages 256 pixels x C halves in shared memory with fully coalesced 16-byte loads (consecutive threads read
-// consecutive chunks of the NHWC stream), rows padded by 16 bytes so that the per-pixel 16-byte reads that follow are
-// bank-conflict free; each thread then owns one pixel; the tiny weight matrix is broadcast from shared memory and the
-// plane writes are coalesced.
-constexpr int kHeadPix = 256;
-__global__ void __launch_bounds__(kHeadPix) pointwise_head_kernel(const __half* __restrict__ in, long npix, int C,
-                                                                  const float* __restrict__ w,
-                                                                  const float* __restrict__ b, int n_out,
-                                                                  float* __restrict__ out, int HW) {
-  extern __shared__ __align__(16) unsigned char head_smem[];
-  float* hw_s = reinterpret_cast<float*>(head_smem);  // [n_out][C] + [n_out] (+ pad to 16 bytes)
-  const int wfloats = (n_out * C + n_out + 3) & ~3;
-  uint4* rows = reinterpret_cast<uint4*>(hw_s + wfloats);  // [kHeadPix][C/8 + 1]
-  const int cpp = C / 8, pitch = cpp + 1;
-  for (int i = threadIdx.x; i < n_out * C; i += blockDim.x) hw_s[i] = w[i];
-  for (int i = threadIdx.x; i < n_out; i += blockDim.x) hw_s[n_out * C + i] = b[i];
-  for (long p0 = (long)blockIdx.x * kHeadPix; p0 < npix; p0 += (long)gridDim.x * kHeadPix) {
-    __syncthreads();  // weights staged / previous tile consumed
-    const long left = npix - p0;
-    const int npx = left < kHeadPix ? (int)left : kHeadPix;
-    const uint4* src = reinterpret_cast<const uint4*>(in + p0 * C);
-    for (int i = threadIdx.x; i < npx * cpp; i += blockDim.x) {
-      const int px = i / cpp, part = i - px * cpp;
-      rows[px * pitch + part] = __ldg(src + i);
-    }
-    __syncthreads();
-    if ((int)threadIdx.x < npx) {
-      float acc[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) acc[j] = (j < n_out) ? hw_s[n_out * C + j] : 0.f;
-      const uint4* ip = rows + threadIdx.x * pitch;
-      for (int c8 = 0; c8 < cpp; ++c8) {
-        const uint4 v = ip[c8];
-        const __half2* h2 = reinterpret_cast<const __half2*>(&v);
-        float x[8];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float2 f = __half22float2(h2[q]);
-          x[2 * q] = f.x;
-          x[2 * q + 1] = f.y;
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          if (j < n_out) {
-            const float4 wa = *reinterpret_cast<const float4*>(hw_s + j * C + c8 * 8);
-            const float4 wb = *reinterpret_cast<const float4*>(hw_s + j * C + c8 * 8 + 4);
-            acc[j] = fmaf(wa.x, x[0], fmaf(wa.y, x[1], fmaf(wa.z, x[2], fmaf(wa.w, x[3], acc[j]))));
-            acc[j] = fmaf(wb.x, x[4], fmaf(wb.y, x[5], fmaf(wb.z, x[6], fmaf(wb.w, x[7], acc[j]))));
-          }
-        }
-      }
-      const long p = p0 + threadIdx.x;
-      const long n = p / HW;
-      const int pix = (int)(p - n * HW);
-      float* o = out + n * (long)n_out * HW + pix;
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        if (j < n_out) o[(long)j * HW] = 1.f / (1.f + __expf(-acc[j]));
-    }
-  }
-}
-
 static int grid_for(long total, int threads) {
   long b = (total + threads - 1) / threads;
   const long cap = (long)num_sms() * 16;
@@ -182,37 +99,6 @@ int launch_maxpool2(const void* in, int N, int H, int W, int C, int c_off, int c
   PB_CUDA(launch_pdl(maxpool2_kernel, dim3(grid_for(total, 256)), dim3(256), 0, s, 1,
                      reinterpret_cast<const __half*>(in), N, H, W, C, c_off, c / 8, reinterpret_cast<__half*>(out), out_C,
                      out_coff));
-  count_launch();
-  return 0;
-}
-
-int launch_upsample2(const void* in, int N, int H, int W, int C, int c_off, int c, void* out, int out_C,
-                     int out_coff, cudaStream_t s) {
-  PB_CHECK(c % 8 == 0 && c_off % 8 == 0 && C % 8 == 0 && out_C % 8 == 0 && out_coff % 8 == 0,
-           "upsample2: channel slices must be multiples of 8");
-  const long total = (long)N * (H * 2) * (W * 2) * (c / 8);
-  PB_CUDA(launch_pdl(upsample2_kernel, dim3(grid_for(total, 256)), dim3(256), 0, s, 1,
-                     reinterpret_cast<const __half*>(in), N, H, W, C, c_off, c / 8, reinterpret_cast<__half*>(out), out_C,
-                     out_coff));
-  count_launch();
-  return 0;
-}
-
-int launch_pointwise_head(const void* in, int N, int H, int W, int C, const float* w, const float* b, int n_out,
-                          float* out, cudaStream_t st) {
-  PB_CHECK(in && w && b && out, "pointwise_head: null pointer");
-  PB_CHECK(C % 8 == 0 && n_out >= 1 && n_out <= 8, "pointwise_head: C %% 8 == 0 and n_out <= 8 required");
-  const long npix = (long)N * H * W;
-  const size_t wfloats = (size_t)((n_out * C + n_out + 3) & ~3);
-  const size_t smem = wfloats * sizeof(float) + (size_t)kHeadPix * (C / 8 + 1) * sizeof(uint4);
-  PB_CHECK(smem <= 96 * 1024, "pointwise_head: C = %d too wide for the staged tile", C);
-  PB_CUDA((cudaError_t)ensure_dynamic_smem(reinterpret_cast<const void*>(pointwise_head_kernel), smem));
-  long blocks = (npix + kHeadPix - 1) / kHeadPix;
-  const long cap = (long)num_sms() * 5;
-  if (blocks > cap) blocks = cap;
-  pointwise_head_kernel<<<(int)blocks, kHeadPix, smem, st>>>(reinterpret_cast<const __half*>(in), npix, C, w, b, n_out,
-                                                            out, H * W);
-  PB_CUDA(cudaGetLastError());
   count_launch();
   return 0;
 }

@@ -145,7 +145,6 @@ __device__ __forceinline__ void epilogue_store16(const ConvKParams& kp, const Ep
 // while chunk i is activated, packed and stored -- and across the S sub-tiles of a halo tile.
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ bool epilogue_fast_ok(const ConvKParams& kp) {
-  if ((kp.dbg_flags & 2) != 0 && kp.out2_mode == PB_OUT2_NONE) return false;
   if (kp.head_n != 0 || (kp.res != nullptr && ((kp.res_C | kp.res_coff) & 7) != 0)) return false;
   if ((reinterpret_cast<uintptr_t>(kp.out) & 31) != 0) return false;  // 32-byte stores
   if (kp.out_mode == PB_OUT_F16_NHWC || kp.out_mode == PB_OUT_F16_NHWC_UP2)
@@ -161,7 +160,6 @@ __device__ __forceinline__ bool epilogue_fast_ok(const ConvKParams& kp) {
 // idle FMA pipe, with the same few-ulp fp32 accuracy (no approximation of the function itself).
 // The exponent is clamped to 2^30 so that the product of four stays finite (< 2^121); silu(v) for v < -20.8 is below
 // 2e-8 in magnitude either way, i.e. an fp16 zero / smallest subnormal.
-// PADEL_B200_CONV_DEBUG bit 0 selects the plain two-MUFU form for A/B runs.
 __device__ __forceinline__ void silu4(float& a, float& b, float& c, float& d) {
   constexpr float kNegLog2e = -1.4426950408889634f;
   const float da = 1.f + ex2_approx(fminf(a * kNegLog2e, 30.f));
@@ -205,7 +203,7 @@ __device__ __forceinline__ void epi_add_res16(const uint4 (&rv)[2], float (&v)[1
 }
 
 // has_res: 0 none, 1 residual after the activation, 2 residual before it (CTA-uniform)
-__device__ __forceinline__ void epi_compute16(int act, int has_res, bool plain_silu, uint32_t (&r)[16],
+__device__ __forceinline__ void epi_compute16(int act, int has_res, uint32_t (&r)[16],
                                               const float* __restrict__ sbias, const uint4 (&rv)[2], float (&v)[16]) {
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
@@ -217,13 +215,8 @@ __device__ __forceinline__ void epi_compute16(int act, int has_res, bool plain_s
   }
   if (has_res == 2) epi_add_res16(rv, v);
   if (act == PB_ACT_SILU) {  // CTA-uniform
-    if (plain_silu) {
 #pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = __fdividef(v[i], 1.f + __expf(-v[i]));
-    } else {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) silu4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
-    }
+    for (int i = 0; i < 4; ++i) silu4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
   } else if (act == PB_ACT_RELU) {
 #pragma unroll
     for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], 0.f);
@@ -234,11 +227,11 @@ __device__ __forceinline__ void epi_compute16(int act, int has_res, bool plain_s
   if (has_res == 1) epi_add_res16(rv, v);
 }
 
-__device__ __forceinline__ void epi_chunk(int act, int has_res, bool plain_silu, const EpiOut& eo, uint32_t (&r)[16],
+__device__ __forceinline__ void epi_chunk(int act, int has_res, const EpiOut& eo, uint32_t (&r)[16],
                                           const float* __restrict__ sbias, char* op, const uint4 (&rv)[2], bool valid,
                                           int nvalid, char* op2 = nullptr, bool vec_tail = false) {
   float v[16];
-  epi_compute16(act, has_res, plain_silu, r, sbias, rv, v);
+  epi_compute16(act, has_res, r, sbias, rv, v);
   if (eo.mode == PB_OUT_F32_NHWC) {
     if (!valid) return;
     if (nvalid >= 16) {
@@ -327,7 +320,6 @@ __device__ __forceinline__ void epilogue_fast(const ConvKParams& kp, const EpiOu
                   : kEpi == PB_EPI_F32                             ? PB_ACT_NONE
                                                                    : kp.act;
   const int has_res = kEpi == PB_EPI_SILU_RES ? 1 : kSpec ? 0 : (kp.res != nullptr ? (kp.res_first ? 2 : 1) : 0);
-  const bool plain_silu = kSpec ? false : (kp.dbg_flags & 1) != 0;
   const int cbytes = eo.mode == PB_OUT_F32_NHWC ? 64 : 32;  // bytes of one 16-channel chunk in the output
   int j = 0, c = 0;
   tmem_ld16(t_addr0, ra);
@@ -364,7 +356,7 @@ __device__ __forceinline__ void epilogue_fast(const ConvKParams& kp, const EpiOu
     }                                                                                                   \
     tmem_ld_wait16(cur);                                                                                \
     if (more) tmem_ld16(t_addr0 + (uint32_t)jn * sub_cols + (uint32_t)(cn * 16), nxt);                  \
-    epi_chunk(act, has_res, plain_silu, eo, cur, sbias + c * 16, op0 + (size_t)j * sub_out + (size_t)(c * cbytes), kPrefetchRes ? rvc : rvl, valid, \
+    epi_chunk(act, has_res, eo, cur, sbias + c * 16, op0 + (size_t)j * sub_out + (size_t)(c * cbytes), kPrefetchRes ? rvc : rvl, valid, \
               cout_n - c * 16, op20 + (size_t)j * sub_out2 + (size_t)(c * 32), kEpi == PB_EPI_F32);      \
     if (!more) break;                                                                                   \
     j = jn;                                                                                             \

@@ -403,21 +403,79 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 // host: geometry + tensor maps for the halo variant. Returns 0 and sets plan->variant = 1 when applicable,
 // returns -1 (no error) when the layer should use the per-tap kernel.
 // ------------------------------------------------------------------------------------------------------------
+constexpr size_t kHaloBudget = 196 * 1024;  // halo + weight rings of a CTA that has the SM to itself
+constexpr size_t kHalfSm = 108 * 1024;      // the whole footprint of one of two CTAs per SM
 
-// Final launch configuration shared by the halo and stem set-ups: two CTAs per SM when the tile fits in half an SM's
-// shared memory and 256 TMEM columns (light n-scale YOLO layers), else one CTA per SM with up to three epilogue groups.
+// TMA swizzle of K-major rows of 128 / 64 / 32 bytes: the swizzle span is the row
+static CUtensorMapSwizzle swizzle_for(uint32_t row_bytes) {
+  return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+         : row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
+                           : CU_TENSOR_MAP_SWIZZLE_32B;
+}
+
+int conv_weight_tmap(CUtensorMap* map, EncodeTiledFn encode, const pb_conv_desc* d, int taps, int box_k, int box_n,
+                     int box_taps) {
+  const cuuint64_t dims[3] = {(cuuint64_t)d->cin, (cuuint64_t)d->cout_pad, (cuuint64_t)taps};
+  const cuuint64_t strides[2] = {(cuuint64_t)d->cin * 2, (cuuint64_t)d->cin * d->cout_pad * 2};
+  const cuuint32_t box[3] = {(cuuint32_t)box_k, (cuuint32_t)box_n, (cuuint32_t)box_taps};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims, strides, box,
+                            estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for((uint32_t)box_k * 2u),
+                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  PB_CHECK(r == CUDA_SUCCESS, "conv: cuTensorMapEncodeTiled(W) failed with %d (cin %d, cout_pad %d, %d taps)", (int)r,
+           d->cin, d->cout_pad, taps);
+  return 0;
+}
+
+int conv_act_tmap(CUtensorMap* map, EncodeTiledFn encode, const pb_conv_desc* d, int s, int box_c, int box_w,
+                  int box_s, int box_h, int box_n) {
+  const cuuint64_t C = (cuuint64_t)d->C, W = (cuuint64_t)d->W, H = (cuuint64_t)d->H, S = (cuuint64_t)s;
+  const cuuint64_t dims[5] = {S * C, W / S, S, H / S, (cuuint64_t)d->N};
+  const cuuint64_t strides[4] = {S * C * 2, W * C * 2, S * W * C * 2, H * W * C * 2};
+  const cuuint32_t box[5] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_s, (cuuint32_t)box_h,
+                             (cuuint32_t)box_n};
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides, box, estr,
+                            CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for((uint32_t)box_c * 2u),
+                            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  PB_CHECK(r == CUDA_SUCCESS, "conv: cuTensorMapEncodeTiled(A) failed with %d (N=%d H=%d W=%d C=%d s=%d)", (int)r, d->N,
+           d->H, d->W, d->C, s);
+  return 0;
+}
+
+// Halo ring next to a resident filter bank of res_total bytes (b_stages = kblocks fixed slots): whatever shared memory is
+// left goes to halo buffers, 2 .. kHaloMaxA.  A light tile (set_cols = S * acc_cols TMEM columns per accumulator set)
+// whose bank and two halo buffers fit in half an SM is sized for half an SM, so two CTAs can share one
+// (halo_finish_config).
+static int halo_resident_a_stages(const ConvKParams& kp, size_t res_total, int set_cols) {
+  const bool small = (size_t)2 * kp.a_bytes + res_total + sizeof(HaloSmemTail) + 1024 <= kHalfSm && set_cols * 2 <= 256;
+  const size_t budget = small ? kHalfSm - sizeof(HaloSmemTail) - 1024 : kHaloBudget;
+  int as = (int)((budget - res_total) / kp.a_bytes);
+  if (as > kHaloMaxA) as = kHaloMaxA;
+  if (as > 2 * kp.kblocks + 1) as = 2 * kp.kblocks + 1;
+  return as < 2 ? 2 : as;
+}
+
+// Tiles, accumulator ring and launch configuration, shared by the halo and stem set-ups once they have set BN, hs_S,
+// pair and the rings.  A tile is 16 output rows (32 for a CTA pair: 16 per CTA) x 8S columns of one image, S
+// accumulator sets of acc_cols TMEM columns.  Two CTAs per SM when the CTA fits in half an SM's shared memory and 256
+// TMEM columns and there are more tiles than SMs (light n-scale YOLO layers), else one CTA per SM with up to three
+// epilogue groups.
 static void halo_finish_config(ConvPlan* plan) {
   ConvKParams& kp = plan->kp;
+  const int S = kp.hs_S;
+  kp.acc_cols = (kp.BN + 31) / 32 * 32;
+  kp.acc_stages = 512 / (S * kp.acc_cols);
+  if (kp.acc_stages > kConvMaxAcc) kp.acc_stages = kConvMaxAcc;
+  kp.idesc = kp.pair ? umma_idesc_f16_m256(kp.BN) : umma_idesc_f16(kp.BN, 0);
+  kp.tiles_w = (kp.Wo + 8 * S - 1) / (8 * S);
+  kp.tiles_h = kp.pair ? (kp.Ho + 31) / 32 : (kp.Ho + 15) / 16;
+  kp.tiles_n = kp.N;
+  kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n;
+
   const size_t need = (size_t)kp.a_stages * kp.a_bytes + (size_t)kp.b_stages * kp.b_bytes + sizeof(HaloSmemTail) + 1024;
-  const int occ_mode = conv_occ_mode();
-  const int set_cols = kp.hs_S * kp.acc_cols;
-  // Half-SM footprint (224 threads, <= 110 KB, 256 TMEM columns): (a) light layers with many tiles run two CTAs of the
-  // SAME kernel per SM; (b) tiny layers (at most two tiles per SM) take it so that CTAs of CONSECUTIVE kernels can be
-  // co-resident -- with programmatic dependent launch the successor then sits through its launch latency (~10 us from
-  // trigger to release, profiles/r02_chain_timeline.txt) while this kernel still computes.
-  const bool tiny = kp.total_tiles <= 2 * num_sms();
-  const bool occ2 = !kp.pair && occ_mode != 0 && need <= 110 * 1024 &&
-                    ((set_cols * 2 <= 256 && kp.total_tiles > num_sms()) || (occ_mode == 2 && tiny && set_cols <= 256));
+  const int set_cols = S * kp.acc_cols;
+  const bool occ2 = !kp.pair && need <= 110 * 1024 && set_cols * 2 <= 256 && kp.total_tiles > num_sms();
   plan->smem_bytes = need;
   if (occ2) {
     if (kp.acc_stages * set_cols > 256) kp.acc_stages = 256 / set_cols;
@@ -436,12 +494,15 @@ static void halo_finish_config(ConvPlan* plan) {
       plan->grid = 2 * pairs;
     }
   }
+  plan->variant = 1;
 }
 
-// Stem (PB_IN_STEM4): 3x3 stride-2 conv over the padded 4-channel input. One TMA box of overlapping 16-element rows
-// (4 pixels x 4 channels, consecutive rows 2 pixels apart) holds, for a tile of 16 x 8S outputs, the three filter
-// rows r = 0..2 as [oh][r][ow] rows of 32 bytes; filter row r of sub-tile j starts at row (r*8S + 8j), 8-row groups
-// (consecutive oh) are 3*8S rows apart.  K = 16 per filter row (12 real), 3 UMMAs per sub-tile.
+// Stem (PB_IN_STEM4): 3x3 stride-2 conv over the padded 4-channel input, K = 16 per filter row (12 real), 3 UMMAs per
+// sub-tile.  The tile's input region -- 34 rows x (16 S + 2) pixels of 8 bytes, every byte once -- is one dense TMA box,
+// and the UMMA descriptor reads the im2col rows out of it: output pixel ow's K = 16 row (pixels 2ow .. 2ow+3) starts 16
+// bytes after its neighbour's, so in the un-swizzled K-major layout (16-byte rows at a 16-byte pitch, second half of a
+// row LBO = 16 bytes on) the overlapping rows ARE the canonical core matrix; the next output row is two image rows
+// further (SBO), filter row r one image row (descriptor offset).
 int conv_stem_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode) {
   PB_CHECK(d->ksize == 3 && d->stride == 2 && d->C == 4 && d->cin == 16 && d->c_in_off == 0,
            "conv(stem): needs ksize 3, stride 2, C = 4, cin = 16");
@@ -451,6 +512,8 @@ int conv_stem_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
   const int acc_cols = (BN + 31) / 32 * 32;
   int S = 4;
   while (S > 1 && (S * acc_cols * 2 > 512)) S >>= 1;
+  const uint32_t pairs = (uint32_t)(8 * S) + 1;  // pixel pairs (16 bytes) per image row of the region
+  const uint32_t pitch = pairs * 16u;
   kp.KB = 16;
   kp.kblocks = 1;
   kp.taps = 3;
@@ -458,105 +521,55 @@ int conv_stem_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
   kp.hs_P = 8 * S;
   kp.hs_G = 3;
   kp.hs_ntaps = 3;
-  kp.hs_sbo_rows = 3 * 8 * S;
+  kp.hs_sbo_rows = (int)(2u * pitch / 16u);  // x hs_a_row_bytes = 2 image rows
   kp.hs_x0 = 0;
   kp.hs_y0 = 0;
-  for (int r = 0; r < 3; ++r) kp.hs_tap_off[r] = r * 8 * S;
-  for (int r = 0; r < 3; ++r) kp.hs_tap_desc[r] = (kp.hs_tap_off[r] * 32) >> 4;
+  for (int r = 0; r < 3; ++r) {
+    kp.hs_tap_off[r] = r * 8 * S;
+    kp.hs_tap_desc[r] = (int)(((uint32_t)r * pitch) >> 4);
+  }
   kp.BN = BN;
   kp.n_ntiles = 1;
-  kp.halo_bytes = 16u * 3u * (uint32_t)(8 * S) * 32u;
-  kp.hs_a_row_bytes = 32u;
-  // Raw-pixel operand (default; PADEL_B200_STEM_RAW=0 selects the overlapping-row box above): the tile's input region --
-  // 34 rows x (16 S + 2) pixels of 8 bytes, every byte once -- is one dense TMA box, and the UMMA descriptor reads the
-  // im2col rows out of it: output pixel ow's K = 16 row (pixels 2ow .. 2ow+3) starts 16 bytes after its neighbour's, so
-  // in the un-swizzled K-major layout (16-byte rows at a 16-byte pitch, second half of a row LBO = 16 bytes on) the
-  // overlapping rows ARE the canonical core matrix; the next output row is two image rows further (SBO), filter row r
-  // one image row (descriptor offset).  A third of the L2->SM traffic and of the shared memory of the box-per-row form.
-  const uint32_t pairs = (uint32_t)(8 * S) + 1;  // pixel pairs (16 bytes) per image row of the region
-  const uint32_t pitch = pairs * 16u;
-  static const int raw = [] {
-    const char* e = getenv("PADEL_B200_STEM_RAW");
-    return e ? atoi(e) : 1;
-  }();
-  if (raw) {
-    kp.halo_bytes = 17u * 2u * pitch;  // 17 row pairs (2 * 16 + 1 rows are read, the 34th is never addressed)
-    kp.hs_a_row_bytes = 16u;
-    kp.hs_sbo_rows = (int)(2u * pitch / 16u);  // x hs_a_row_bytes = 2 image rows
-    for (int r = 0; r < 3; ++r) kp.hs_tap_desc[r] = (int)(((uint32_t)r * pitch) >> 4);
-  }
+  kp.halo_bytes = 17u * 2u * pitch;  // 17 row pairs (2 * 16 + 1 rows are read, the 34th is never addressed)
+  kp.hs_a_row_bytes = 16u;
   kp.a_bytes = (kp.halo_bytes + 1023u) & ~1023u;
   kp.b_tx_bytes = 3u * (uint32_t)BN * 32u;
   kp.b_bytes = (kp.b_tx_bytes + 1023u) & ~1023u;
   kp.a_stages = 4;
   kp.b_stages = 1;  // the three filter rows are one small box: resident
   kp.b_resident = 1;
-  kp.acc_cols = acc_cols;
-  kp.acc_stages = 512 / (S * acc_cols);
-  if (kp.acc_stages > kConvMaxAcc) kp.acc_stages = kConvMaxAcc;
-  kp.idesc = umma_idesc_f16(BN, 0);
-  kp.tiles_w = (kp.Wo + 8 * S - 1) / (8 * S);
-  kp.tiles_h = (kp.Ho + 15) / 16;
-  kp.tiles_n = kp.N;
-  kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n;
   halo_finish_config(plan);
-  plan->variant = 1;
   {
-    // overlapping-row view of the padded (N, H+2, W+2, 4) tensor: element (k, ow, r, oh, n) =
-    //   base + n*(H+2)*(W+2)*8 + (2*oh + r)*(W+2)*8 + (2*ow)*8 + 2*k  -> pixels 2ow-1 .. 2ow+2 of image row 2oh+r-1
+    // dense view (pixel pair, image-row parity, image-row pair) of the padded (N, H+2, W+2, 4) tensor: element
+    // (k, p, q, y, n) = base + n*Hp*Wp*8 + (2*y + q)*Wp*8 + p*16 + 2*k; the producer's coordinates (0, ow0, 0, oh0, n)
+    // address pixel pair ow0 = pixel 2*ow0 and image row 2*oh0 of the padded tensor, i.e. the tile's top-left tap
     const cuuint64_t Wp = (cuuint64_t)d->W + 2, Hp = (cuuint64_t)d->H + 2;
-    cuuint64_t dims[5] = {16, (cuuint64_t)d->W / 2, 3, (cuuint64_t)d->H / 2, (cuuint64_t)d->N};
-    cuuint64_t strides[4] = {16, Wp * 8, 2 * Wp * 8, Hp * Wp * 8};
-    cuuint32_t box[5] = {16, (cuuint32_t)(8 * S), 3, 16, 1};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_32B;
-    if (raw) {
-      // dense view (pixel pair, image-row parity, image-row pair): element (k, p, q, y, n) =
-      //   base + n*Hp*Wp*8 + (2*y + q)*Wp*8 + p*16 + 2*k; the producer's coordinates (0, ow0, 0, oh0, n) address
-      //   pixel pair ow0 = pixel 2*ow0 and image row 2*oh0 of the padded tensor, i.e. the tile's top-left tap
-      dims[0] = 8, dims[1] = Wp / 2, dims[2] = 2, dims[3] = Hp / 2;
-      strides[0] = 16, strides[1] = Wp * 8, strides[2] = 2 * Wp * 8;
-      box[0] = 8, box[1] = pairs, box[2] = 2, box[3] = 17;
-      swz = CU_TENSOR_MAP_SWIZZLE_NONE;
-    }
-    CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides,
-                        box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(stem): cuTensorMapEncodeTiled(A, overlapping rows) failed with %d", (int)r);
+    const cuuint64_t dims[5] = {8, Wp / 2, 2, Hp / 2, (cuuint64_t)d->N};
+    const cuuint64_t strides[4] = {16, Wp * 8, 2 * Wp * 8, Hp * Wp * 8};
+    const cuuint32_t box[5] = {8, pairs, 2, 17, 1};
+    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    const CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims,
+                              strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    PB_CHECK(r == CUDA_SUCCESS, "conv(stem): cuTensorMapEncodeTiled(A) failed with %d", (int)r);
   }
-  {
-    cuuint64_t dims[3] = {16, (cuuint64_t)d->cout_pad, 3};
-    cuuint64_t strides[2] = {32, (cuuint64_t)d->cout_pad * 32};
-    cuuint32_t box[3] = {16, (cuuint32_t)BN, 3};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims,
-                        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(stem): cuTensorMapEncodeTiled(W) failed with %d", (int)r);
-  }
-  return 0;
+  return conv_weight_tmap(&plan->tmap_w, encode, d, 3, 16, BN, 3);
 }
 
 int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode) {
   if (d->ksize != 3 || d->stride != 1 || d->cout_pad > 256) return -1;
-  ConvKParams& kp = plan->kp;  // common fields (epilogue, KB, kblocks, idesc, ...) already filled by the caller
+  ConvKParams& kp = plan->kp;  // common fields (epilogue, KB, kblocks, ...) already filled by the caller
   const int BN = d->cout_pad;
   const uint32_t row_bytes = (uint32_t)kp.KB * 2u;
   const int acc_cols = (BN + 31) / 32 * 32;
-  const size_t budget = 196 * 1024;
   // Choose S (sub-tiles per CTA tile: fewer halo + weight bytes per pixel) first, then G (taps per weight box:
   // fewer TMA operations) as large as shared memory allows.
   const uint32_t tap_bytes = (uint32_t)BN * row_bytes;
   // Resident filter bank: all nine taps of every channel block (one box per block) stay in shared memory for the
   // whole kernel when they fit next to two halo buffers; otherwise weight boxes are streamed through a ring.
-  // PADEL_B200_CONV_BRES=0 disables (A/B testing).
   const uint32_t res_box = (9u * tap_bytes + 1023u) & ~1023u;
   const size_t res_total = (size_t)kp.kblocks * res_box;
-  bool resident = false;
-  {
-    const char* er = getenv("PADEL_B200_CONV_BRES");
-    resident = (!er || atoi(er) != 0) && kp.kblocks <= kHaloMaxB && res_total <= 120 * 1024;
-  }
+  bool resident = kp.kblocks <= kHaloMaxB && res_total <= 120 * 1024;
   int bestS = 0, best_cols = 0, G = 1;
   for (int pass = resident ? 0 : 1; pass < 2 && bestS == 0; ++pass) {
     resident = resident && pass == 0;
@@ -566,12 +579,12 @@ int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
       const uint32_t a_alloc = (halo + 1023u) & ~1023u;
       int g_fit = 0;
       if (resident) {
-        if ((size_t)2 * a_alloc + res_total <= budget) g_fit = 9;
+        if ((size_t)2 * a_alloc + res_total <= kHaloBudget) g_fit = 9;
       } else {
         for (int g = 9; g >= 1; g = (g == 9 ? 3 : (g == 3 ? 1 : 0))) {
           const uint32_t ba = ((uint32_t)g * tap_bytes + 1023u) & ~1023u;
           const int min_b = g == 9 ? 2 : (g == 3 ? 3 : 4);
-          if ((size_t)2 * a_alloc + (size_t)min_b * ba <= budget) {
+          if ((size_t)2 * a_alloc + (size_t)min_b * ba <= kHaloBudget) {
             g_fit = g;
             break;
           }
@@ -594,18 +607,16 @@ int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
   // weights.  Measured on TrackNet at batch 32 (profiles/r01_layers.txt): the deep-K narrow layers gain (192->64:
   // 935 -> 757 us = 1.38 PFLOP/s, above the ~1.27 PFLOP/s a single CTA can issue at N = 64; 384->128: 768 -> 676 us;
   // 128->128: 269 -> 231 us), shallow-K layers (cin <= 64) and the 2x2-replicating stores lose a few percent.
-  // Default rule: cin >= 128, plain fp16 store, enough tiles to fill the machine with pairs.
-  // PADEL_B200_CONV_PAIR=0/1 forces it off / on wherever it applies.
+  // Rule: cin >= 128, plain fp16 store, enough tiles to fill the machine with pairs (unless overridden).
   {
-    const char* ep = getenv("PADEL_B200_CONV_PAIR");
-    const int pm = ep ? atoi(ep) : 2;
+    const int pm = conv_override("PADEL_B200_CONV_PAIR");
     const bool can = BN % 32 == 0 && BN >= 32 && kp.Ho >= 32;
     const long pair_tiles = (long)((d->W + 8 * S - 1) / (8 * S)) * ((kp.Ho + 31) / 32) * kp.N;
     const bool want = d->cin >= 128 && d->out_mode == PB_OUT_F16_NHWC && pair_tiles >= 2L * (num_sms() / 2);
     kp.pair = (can && (pm == 1 || (pm == 2 && want))) ? 1 : 0;
     if (kp.pair && resident) {  // forced pair mode: stream the weights (each CTA holds half of them)
       resident = false;
-      if (G == 9 && (size_t)2 * (((18u * (uint32_t)(8 * bestS + 2) * row_bytes) + 1023u) & ~1023u) + (size_t)2 * b_alloc > budget)
+      if (G == 9 && (size_t)2 * (((18u * (uint32_t)(8 * bestS + 2) * row_bytes) + 1023u) & ~1023u) + (size_t)2 * b_alloc > kHaloBudget)
         return -1;
     }
   }
@@ -631,72 +642,29 @@ int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
   kp.b_bytes = b_alloc;
   kp.a_stages = 2;
   if (resident) {
-    // the filter bank occupies kblocks fixed slots; whatever is left goes to halo buffers (up to kHaloMaxA)
     kp.b_stages = kp.kblocks;
-    const bool tiny_mode = conv_occ_mode() == 2 && !kp.pair &&
-                           (long)((kp.Wo + 8 * S - 1) / (8 * S)) * ((kp.Ho + 15) / 16) * kp.N <= 2L * num_sms();
-    const bool small = (size_t)2 * kp.a_bytes + res_total + sizeof(HaloSmemTail) + 1024 <= 108 * 1024 &&
-                       (S * acc_cols * 2 <= 256 || (tiny_mode && S * acc_cols <= 256));
-    const size_t budget2 = small ? (size_t)108 * 1024 - sizeof(HaloSmemTail) - 1024 : budget;
-    int as = (int)((budget2 - res_total) / kp.a_bytes);
-    if (as > kHaloMaxA) as = kHaloMaxA;
-    if (as > 2 * kp.kblocks + 1) as = 2 * kp.kblocks + 1;
-    kp.a_stages = as < 2 ? 2 : as;
+    kp.a_stages = halo_resident_a_stages(kp, res_total, S * acc_cols);
   } else {
-  // light layers: size the rings for half an SM so that two CTAs can be co-resident (see halo_finish_config)
-  const int min_b_small = G == 9 ? 2 : (G == 3 ? 3 : 4);
-  const bool tiny_mode = conv_occ_mode() == 2 && !kp.pair &&
-                         (long)((kp.Wo + 8 * S - 1) / (8 * S)) * ((kp.Ho + 15) / 16) * kp.N <= 2L * num_sms();
-  const bool small = (size_t)2 * kp.a_bytes + (size_t)min_b_small * b_alloc + sizeof(HaloSmemTail) + 1024 <= 108 * 1024 &&
-                     (S * acc_cols * 2 <= 256 || (tiny_mode && S * acc_cols <= 256));
-  const size_t budget2 = small ? (size_t)108 * 1024 - sizeof(HaloSmemTail) - 1024 : budget;
-  size_t rest = budget2 - (size_t)2 * kp.a_bytes;
-  if (kp.kblocks > 2 && rest > (size_t)kp.a_bytes + 4 * (size_t)b_alloc) {  // a third halo buffer when K is deep
-    kp.a_stages = 3;
-    rest -= kp.a_bytes;
+    // light layers: size the rings for half an SM so that two CTAs can be co-resident (see halo_finish_config)
+    const int min_b_small = G == 9 ? 2 : (G == 3 ? 3 : 4);
+    const bool small =
+        (size_t)2 * kp.a_bytes + (size_t)min_b_small * b_alloc + sizeof(HaloSmemTail) + 1024 <= kHalfSm &&
+        S * acc_cols * 2 <= 256;
+    const size_t budget2 = small ? kHalfSm - sizeof(HaloSmemTail) - 1024 : kHaloBudget;
+    size_t rest = budget2 - (size_t)2 * kp.a_bytes;
+    if (kp.kblocks > 2 && rest > (size_t)kp.a_bytes + 4 * (size_t)b_alloc) {  // a third halo buffer when K is deep
+      kp.a_stages = 3;
+      rest -= kp.a_bytes;
+    }
+    int bs = (int)(rest / b_alloc);
+    if (bs > kHaloMaxB) bs = kHaloMaxB;
+    if (bs > 9 * kp.kblocks / G * 2) bs = 9 * kp.kblocks / G * 2;
+    if (bs < 2) bs = 2;
+    kp.b_stages = bs;
   }
-  int bs = (int)(rest / b_alloc);
-  if (bs > kHaloMaxB) bs = kHaloMaxB;
-  if (bs > 9 * kp.kblocks / G * 2) bs = 9 * kp.kblocks / G * 2;
-  if (bs < 2) bs = 2;
-  kp.b_stages = bs;
-  }
-  kp.acc_cols = acc_cols;
-  kp.acc_stages = 512 / (S * acc_cols);
-  if (kp.acc_stages > kConvMaxAcc) kp.acc_stages = kConvMaxAcc;
-  kp.idesc = kp.pair ? umma_idesc_f16_m256(BN) : umma_idesc_f16(BN, 0);
-  kp.tiles_w = (kp.Wo + 8 * S - 1) / (8 * S);
-  kp.tiles_h = kp.pair ? (kp.Ho + 31) / 32 : (kp.Ho + 15) / 16;
-  kp.tiles_n = kp.N;
-  kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n;
   halo_finish_config(plan);
-  plan->variant = 1;
-
-  const CUtensorMapSwizzle swz = kp.KB == 64   ? CU_TENSOR_MAP_SWIZZLE_128B
-                                 : kp.KB == 32 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                               : CU_TENSOR_MAP_SWIZZLE_32B;
-  {
-    const cuuint64_t C = (cuuint64_t)d->C, W = (cuuint64_t)d->W, H = (cuuint64_t)d->H;
-    cuuint64_t dims[5] = {C, W, 1, H, (cuuint64_t)d->N};
-    cuuint64_t strides[4] = {C * 2, W * C * 2, W * C * 2, H * W * C * 2};
-    cuuint32_t box[5] = {(cuuint32_t)kp.KB, (cuuint32_t)P, 1, 18, 1};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides,
-                        box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo): cuTensorMapEncodeTiled(A) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[3] = {(cuuint64_t)d->cin, (cuuint64_t)d->cout_pad, 9};
-    cuuint64_t strides[2] = {(cuuint64_t)d->cin * 2, (cuuint64_t)d->cin * d->cout_pad * 2};
-    cuuint32_t box[3] = {(cuuint32_t)kp.KB, (cuuint32_t)(kp.pair ? BN / 2 : BN), (cuuint32_t)G};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims,
-                        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo): cuTensorMapEncodeTiled(W) failed with %d", (int)r);
-  }
-  return 0;
+  if (conv_act_tmap(&plan->tmap_a, encode, d, 1, kp.KB, P, 1, 18, 1)) return 1;
+  return conv_weight_tmap(&plan->tmap_w, encode, d, 9, kp.KB, kp.pair ? BN / 2 : BN, G);
 }
 
 // 1x1 / stride-1 layers through the same kernel (one tap, no halo): a CTA tile is 16 rows x 8S columns (up to 512
@@ -705,22 +673,15 @@ int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode)
 // 128-pixel tile, as many bytes as the activations when cin ~ cout, and pays its fixed per-tile costs four times as
 // often.  Measured on the pose program (batch 32, profiles/r02_layers_final.txt): cin 32 -> 32 @320^2 152 -> 93 us; every
 // layer with cin >= 64 is 0-15 % SLOWER than on the per-tap kernel (whose flattened 128-pixel tiles waste nothing at the
-// image edges and whose K loop is deeper).  Default rule therefore: cin <= 32; PADEL_B200_CONV_HALO1=0 disables it, =2
-// takes every 1x1 layer whose bank fits next to two activation buffers.
+// image edges and whose K loop is deeper).  Rule therefore: cin <= 32.
 int conv_halo_1x1_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode) {
-  static const int enabled = [] {
-    const char* e = getenv("PADEL_B200_CONV_HALO1");
-    return e ? atoi(e) : 1;
-  }();
-  if (!enabled || d->ksize != 1 || d->stride != 1 || d->cout_pad > 256 || d->head_n != 0) return -1;
-  if (enabled == 1 && d->cin > 32) return -1;
+  if (d->ksize != 1 || d->stride != 1 || d->cout_pad > 256 || d->head_n != 0 || d->cin > 32) return -1;
   // fp32 outputs (YOLO head maps, the TrackNet predictor) keep the per-tap kernel and its fp32 epilogue class
   if (d->out_mode != PB_OUT_F16_NHWC && d->out_mode != PB_OUT_F16_NHWC_UP2) return -1;
   ConvKParams& kp = plan->kp;  // common fields already filled by the caller
   const int BN = d->cout_pad;
   const uint32_t row_bytes = (uint32_t)kp.KB * 2u;
   const int acc_cols = (BN + 31) / 32 * 32;
-  const size_t budget = 196 * 1024;
   const uint32_t tap_bytes = (uint32_t)BN * row_bytes;
   const uint32_t res_box = (tap_bytes + 1023u) & ~1023u;
   const size_t res_total = (size_t)kp.kblocks * res_box;
@@ -729,7 +690,7 @@ int conv_halo_1x1_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn enc
   for (int s = 4; s >= 1; s >>= 1) {
     if (s * acc_cols * 2 > 512) continue;  // keep >= 2 accumulator sets in TMEM
     const uint32_t a_alloc = (16u * (uint32_t)(8 * s) * row_bytes + 1023u) & ~1023u;
-    if ((size_t)2 * a_alloc + res_total > budget) continue;
+    if ((size_t)2 * a_alloc + res_total > kHaloBudget) continue;
     if (s > 1 && d->W <= 8 * (s / 2)) continue;  // a narrower tile already covers the row
     S = s;
     break;
@@ -755,49 +716,10 @@ int conv_halo_1x1_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn enc
   kp.b_tx_bytes = tap_bytes;
   kp.b_bytes = res_box;
   kp.b_stages = kp.kblocks;
-  {
-    const bool small = (size_t)2 * kp.a_bytes + res_total + sizeof(HaloSmemTail) + 1024 <= 108 * 1024 && S * acc_cols * 2 <= 256;
-    const size_t budget2 = small ? (size_t)108 * 1024 - sizeof(HaloSmemTail) - 1024 : budget;
-    int as = (int)((budget2 - res_total) / kp.a_bytes);
-    if (as > kHaloMaxA) as = kHaloMaxA;
-    if (as > 2 * kp.kblocks + 1) as = 2 * kp.kblocks + 1;
-    kp.a_stages = as < 2 ? 2 : as;
-  }
-  kp.acc_cols = acc_cols;
-  kp.acc_stages = 512 / (S * acc_cols);
-  if (kp.acc_stages > kConvMaxAcc) kp.acc_stages = kConvMaxAcc;
-  kp.idesc = umma_idesc_f16(BN, 0);
-  kp.tiles_w = (kp.Wo + 8 * S - 1) / (8 * S);
-  kp.tiles_h = (kp.Ho + 15) / 16;
-  kp.tiles_n = kp.N;
-  kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n;
+  kp.a_stages = halo_resident_a_stages(kp, res_total, S * acc_cols);
   halo_finish_config(plan);
-  plan->variant = 1;
-  const CUtensorMapSwizzle swz = kp.KB == 64   ? CU_TENSOR_MAP_SWIZZLE_128B
-                                 : kp.KB == 32 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                               : CU_TENSOR_MAP_SWIZZLE_32B;
-  {
-    const cuuint64_t C = (cuuint64_t)d->C, W = (cuuint64_t)d->W, H = (cuuint64_t)d->H;
-    cuuint64_t dims[5] = {C, W, 1, H, (cuuint64_t)d->N};
-    cuuint64_t strides[4] = {C * 2, W * C * 2, W * C * 2, H * W * C * 2};
-    cuuint32_t box[5] = {(cuuint32_t)kp.KB, (cuuint32_t)P, 1, 16, 1};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides,
-                        box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo 1x1): cuTensorMapEncodeTiled(A) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[3] = {(cuuint64_t)d->cin, (cuuint64_t)d->cout_pad, 1};
-    cuuint64_t strides[2] = {(cuuint64_t)d->cin * 2, (cuuint64_t)d->cin * d->cout_pad * 2};
-    cuuint32_t box[3] = {(cuuint32_t)kp.KB, (cuuint32_t)BN, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims,
-                        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo 1x1): cuTensorMapEncodeTiled(W) failed with %d", (int)r);
-  }
-  return 0;
+  if (conv_act_tmap(&plan->tmap_a, encode, d, 1, kp.KB, P, 1, 16, 1)) return 1;
+  return conv_weight_tmap(&plan->tmap_w, encode, d, 1, kp.KB, BN, 1);
 }
 
 // 3x3 / stride-2 conv over a whole C = 16 / 32 channel tensor.  The input is read through the pixel-pair view
@@ -821,12 +743,11 @@ int conv_halo_s2_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn enco
   const int acc_cols = (BN + 31) / 32 * 32;
   const uint32_t tap_bytes = (uint32_t)BN * row_bytes;
   const uint32_t b_alloc = (9u * tap_bytes + 1023u) & ~1023u;  // all nine taps in one weight box
-  const size_t budget = 196 * 1024;
   int S = 0;
   for (int s = 4; s >= 1; s >>= 1) {
     if (s * acc_cols * 2 > 512) continue;
     const uint32_t halo = 34u * (uint32_t)(8 * s + 1) * a_row;
-    if ((size_t)2 * ((halo + 1023u) & ~1023u) + (size_t)2 * b_alloc <= budget) {
+    if ((size_t)2 * ((halo + 1023u) & ~1023u) + (size_t)2 * b_alloc <= kHaloBudget) {
       S = s;
       break;
     }
@@ -860,40 +781,9 @@ int conv_halo_s2_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn enco
   kp.a_stages = 2;
   kp.b_stages = 1;  // all nine taps are one box: resident
   kp.b_resident = 1;
-  kp.acc_cols = acc_cols;
-  kp.acc_stages = 512 / (S * acc_cols);
-  if (kp.acc_stages > kConvMaxAcc) kp.acc_stages = kConvMaxAcc;
-  kp.idesc = umma_idesc_f16(BN, 0);
-  kp.tiles_w = (kp.Wo + 8 * S - 1) / (8 * S);
-  kp.tiles_h = (kp.Ho + 15) / 16;
-  kp.tiles_n = kp.N;
-  kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n;
   halo_finish_config(plan);
-  plan->variant = 1;
-  {
-    const cuuint64_t C = (cuuint64_t)d->C, W = (cuuint64_t)d->W, H = (cuuint64_t)d->H;
-    cuuint64_t dims[5] = {2 * C, W / 2, 2, H / 2, (cuuint64_t)d->N};
-    cuuint64_t strides[4] = {2 * C * 2, W * C * 2, 2 * W * C * 2, H * W * C * 2};
-    cuuint32_t box[5] = {(cuuint32_t)(2 * d->C), (cuuint32_t)P, 2, 17, 1};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides,
-                        box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        a_row == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo s2): cuTensorMapEncodeTiled(A) failed with %d", (int)r);
-  }
-  {
-    cuuint64_t dims[3] = {(cuuint64_t)d->cin, (cuuint64_t)d->cout_pad, 9};
-    cuuint64_t strides[2] = {(cuuint64_t)d->cin * 2, (cuuint64_t)d->cin * d->cout_pad * 2};
-    cuuint32_t box[3] = {(cuuint32_t)d->cin, (cuuint32_t)BN, 9};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims,
-                        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv(halo s2): cuTensorMapEncodeTiled(W) failed with %d", (int)r);
-  }
-  return 0;
+  if (conv_act_tmap(&plan->tmap_a, encode, d, 2, 2 * d->cin, P, 2, 17, 1)) return 1;
+  return conv_weight_tmap(&plan->tmap_w, encode, d, 9, d->cin, BN, 9);
 }
 
 typedef void (*HaloKernelFn)(CUtensorMap, CUtensorMap, ConvKParams);
@@ -925,8 +815,7 @@ int conv_halo_launch(const ConvPlan* plan, cudaStream_t stream) {
   HaloKernelFn fn = halo_kernel_pick(plan);
   PB_CHECK(fn != nullptr, "conv(halo): no kernel instantiation for S=%d, k-steps=%d", kp.hs_S, kp.KB / 16);
   PB_CUDA((cudaError_t)ensure_dynamic_smem(reinterpret_cast<const void*>(fn), 227 * 1024));
-  cudaError_t le = launch_ex(fn, dim3(plan->grid), dim3(plan->threads), plan->smem_bytes, stream, kp.pair ? 2 : 1,
-                              plan->pdl != 0,
+  cudaError_t le = launch_pdl(fn, dim3(plan->grid), dim3(plan->threads), plan->smem_bytes, stream, kp.pair ? 2 : 1,
                               plan->tmap_a, plan->tmap_w, plan->kp);
   PB_CHECK(le == cudaSuccess,
            "conv(halo): launch failed: %s (pair %d, grid %d, threads %d, smem %zu, tiles %d, S %d, BN %d, KB %d)",

@@ -329,12 +329,6 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-static int ilog2(int v) {
-  int l = 0;
-  while ((1 << l) < v) ++l;
-  return l;
-}
-
 #ifdef PB_DEBUG_BUILD  // libpadel_b200_debug.so only: clock64 role timelines of CTA 0 (scripts/exp_timeline*.py)
 static long long* g_conv_dbg = nullptr;
 extern "C" void pb_debug_conv_timeline(long long* buf) { g_conv_dbg = buf; }
@@ -344,13 +338,9 @@ static long long* const g_conv_dbg = nullptr;
 
 // Which epilogue instantiation a layer runs: a plain class when the vectorised epilogue applies (the conditions of
 // epilogue_fast_ok) and the layer is activation-only -- no residual, fp16 NHWC store, no secondary output, no fused head.
-// PADEL_B200_CONV_EPI=0 keeps every layer on the run-time epilogue (A/B).
+// The debug library's role timelines (kp.dbg) are recorded by the run-time epilogue only.
 int conv_epi_class(const pb_conv_desc* d, const ConvKParams& kp) {
-  static const int enabled = [] {
-    const char* e = getenv("PADEL_B200_CONV_EPI");
-    return e ? atoi(e) : 1;
-  }();
-  if (!enabled || kp.dbg_flags != 0 || kp.dbg != nullptr) return PB_EPI_GENERIC;
+  if (kp.dbg != nullptr) return PB_EPI_GENERIC;
   if (d->head_n != 0 || d->out2_mode != PB_OUT2_NONE || (reinterpret_cast<uintptr_t>(d->out) & 31) != 0)
     return PB_EPI_GENERIC;
   if (d->out_mode == PB_OUT_F32_NHWC) {  // 32-byte aligned 8-float groups
@@ -448,19 +438,12 @@ static int conv_plan_build_impl(const pb_conv_desc* d, ConvPlan* plan) {
   kp.head_n = d->head_n;
   kp.head_out = d->head_out;
   kp.dbg = g_conv_dbg;
-  {
-    const char* df = getenv("PADEL_B200_CONV_DEBUG");
-    kp.dbg_flags = df ? atoi(df) : 0;
-  }
   plan->variant = 0;
-  plan->pdl = plan_pdl();
   plan->epi = conv_epi_class(d, kp);
   if (stem) return conv_stem_setup(d, plan, encode);
   {
-    // halo variant for 3x3/s1 layers: default on for cout <= 192 (the layers the per-tap kernel leaves
-    // L2/TMA-bound); PADEL_B200_CONV_HALO=0 disables it, =1 forces it wherever it applies
-    const char* e = getenv("PADEL_B200_CONV_HALO");
-    const int mode = e ? atoi(e) : 2;
+    // halo variant: for cout <= 192 (the layers the per-tap kernel leaves L2/TMA-bound) unless overridden
+    const int mode = conv_override("PADEL_B200_CONV_HALO");
     if (mode == 1 || (mode == 2 && d->cout_pad <= 192)) {
       const int rc = d->ksize == 1    ? conv_halo_1x1_setup(d, plan, encode)
                      : d->stride == 2 ? conv_halo_s2_setup(d, plan, encode)
@@ -497,7 +480,6 @@ static int conv_plan_build_impl(const pb_conv_desc* d, ConvPlan* plan) {
   kp.tiles_h = (kp.Ho + TH - 1) / TH;
   kp.tiles_n = (kp.N + TN - 1) / TN;
   kp.total_tiles = kp.tiles_w * kp.tiles_h * kp.tiles_n * kp.n_ntiles;
-  (void)ilog2;
 
   for (int r = 0; r < d->ksize; ++r)
     for (int q = 0; q < d->ksize; ++q) {
@@ -527,12 +509,8 @@ static int conv_plan_build_impl(const pb_conv_desc* d, ConvPlan* plan) {
   kp.b_bytes = (kp.b_tx_bytes + 1023u) & ~1023u;
   const uint32_t stage_bytes = kp.a_bytes + kp.b_bytes;
   // Two CTAs per SM for light layers (small stages, narrow N): each gets half the shared memory and 256 TMEM
-  // columns, so one CTA's TMA / epilogue latency is covered by the other's work.  PADEL_B200_CONV_OCC2=0 disables.
-  const int occ_mode = conv_occ_mode();
-  const bool tiny = kp.total_tiles <= 2 * num_sms();  // see halo_finish_config: co-residency of consecutive kernels
-  const bool occ2 = occ_mode != 0 &&
-                    (((size_t)stage_bytes * 6 <= 96 * 1024 && kp.acc_cols * 2 <= 256 && kp.total_tiles > num_sms()) ||
-                     (occ_mode == 2 && tiny && (size_t)stage_bytes * 2 <= 96 * 1024 && kp.acc_cols <= 256));
+  // columns, so one CTA's TMA / epilogue latency is covered by the other's work.
+  const bool occ2 = (size_t)stage_bytes * 6 <= 96 * 1024 && kp.acc_cols * 2 <= 256 && kp.total_tiles > num_sms();
   const size_t budget = occ2 ? 96 * 1024 : 200 * 1024;
   int stages = (int)(budget / stage_bytes);
   if (stages > kConvMaxStages) stages = kConvMaxStages;
@@ -552,40 +530,8 @@ static int conv_plan_build_impl(const pb_conv_desc* d, ConvPlan* plan) {
     plan->threads = conv_threads_for(kp.egroups);
     plan->grid = kp.total_tiles < num_sms() ? kp.total_tiles : num_sms();
   }
-  const CUtensorMapSwizzle swz = kp.KB == 64   ? CU_TENSOR_MAP_SWIZZLE_128B
-                                 : kp.KB == 32 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                               : CU_TENSOR_MAP_SWIZZLE_32B;
-  {
-    // activations: stride 1 -> (C, W, 1, H, N); stride 2 -> (2C, W/2, 2, H/2, N)
-    const cuuint64_t C = (cuuint64_t)d->C, W = (cuuint64_t)d->W, H = (cuuint64_t)d->H;
-    cuuint64_t dims[5];
-    cuuint64_t strides[4];
-    if (s == 1) {
-      dims[0] = C; dims[1] = W; dims[2] = 1; dims[3] = H; dims[4] = (cuuint64_t)d->N;
-      strides[0] = C * 2; strides[1] = W * C * 2; strides[2] = W * C * 2; strides[3] = H * W * C * 2;
-    } else {
-      dims[0] = 2 * C; dims[1] = W / 2; dims[2] = 2; dims[3] = H / 2; dims[4] = (cuuint64_t)d->N;
-      strides[0] = 2 * C * 2; strides[1] = W * C * 2; strides[2] = 2 * W * C * 2; strides[3] = H * W * C * 2;
-    }
-    cuuint32_t box[5] = {(cuuint32_t)kp.KB, (cuuint32_t)TW, 1, (cuuint32_t)TH, (cuuint32_t)TN};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = encode(&plan->tmap_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(d->in), dims, strides,
-                        box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv: cuTensorMapEncodeTiled(A) failed with %d (N=%d H=%d W=%d C=%d s=%d)", (int)r,
-             d->N, d->H, d->W, d->C, s);
-  }
-  {
-    cuuint64_t dims[3] = {(cuuint64_t)d->cin, (cuuint64_t)d->cout_pad, (cuuint64_t)kp.taps};
-    cuuint64_t strides[2] = {(cuuint64_t)d->cin * 2, (cuuint64_t)d->cin * d->cout_pad * 2};
-    cuuint32_t box[3] = {(cuuint32_t)kp.KB, (cuuint32_t)kp.BN, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = encode(&plan->tmap_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d->weight), dims,
-                        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    PB_CHECK(r == CUDA_SUCCESS, "conv: cuTensorMapEncodeTiled(W) failed with %d", (int)r);
-  }
-  return 0;
+  if (conv_act_tmap(&plan->tmap_a, encode, d, s, kp.KB, TW, 1, TH, TN)) return 1;
+  return conv_weight_tmap(&plan->tmap_w, encode, d, kp.taps, kp.KB, kp.BN, 1);
 }
 
 int conv_plan_build(const pb_conv_desc* d, ConvPlan* plan) {
@@ -607,8 +553,8 @@ int conv_plan_launch(const ConvPlan* plan, cudaStream_t stream) {
                         : plan->epi == PB_EPI_F32      ? conv_tc_kernel<PB_EPI_F32>
                                                        : conv_tc_kernel<PB_EPI_GENERIC>;
   PB_CUDA((cudaError_t)ensure_dynamic_smem(reinterpret_cast<const void*>(fn), 227 * 1024));
-  PB_CUDA(launch_ex(fn, dim3(plan->grid), dim3(plan->threads), plan->smem_bytes, stream, 1, plan->pdl != 0, plan->tmap_a,
-                    plan->tmap_w, plan->kp));
+  PB_CUDA(launch_pdl(fn, dim3(plan->grid), dim3(plan->threads), plan->smem_bytes, stream, 1, plan->tmap_a, plan->tmap_w,
+                     plan->kp));
   count_launch();
   return 0;
 }

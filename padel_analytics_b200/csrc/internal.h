@@ -17,20 +17,18 @@ namespace pb {
 void set_error(const char* fmt, ...);
 extern std::atomic<long long> g_launches;
 inline void count_launch(int n = 1) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-int num_sms();
+int num_sms();  // streaming multiprocessors of the current device
 // Raise a kernel's dynamic shared-memory limit to at least `bytes` on the CURRENT device (the attribute is per device
 // and per function; remembered per (device, function) so the driver call happens once).  Returns a cudaError_t.
 int ensure_dynamic_smem(const void* func, size_t bytes);
-// Programmatic dependent launch for the kernels of a program (PADEL_B200_PDL=0 disables; default on)
-bool pdl_enabled();
-int plan_pdl();  // the value a plan built now captures
 
 #ifdef __CUDACC__
-// Launch `kernel` with the programmatic-stream-serialization attribute (see ptx.cuh::griddep_wait): only for kernels
-// that call griddep_wait() before touching data another kernel may have written / may still be reading.
+// Launch `kernel` with programmatic dependent launch (the programmatic-stream-serialization attribute, see
+// ptx.cuh::griddep_wait) and, for cluster > 1, as clusters of that many CTAs: only for kernels that call griddep_wait()
+// before touching data another kernel may have written / may still be reading.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                             int cluster, bool pdl, Args... args) {
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                              int cluster, Args... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
@@ -45,21 +43,13 @@ inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
     attr[na].val.clusterDim.z = 1;
     ++na;
   }
-  if (pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
+  attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[na].val.programmaticStreamSerializationAllowed = 1;
+  ++na;
   cfg.attrs = attr;
   cfg.numAttrs = (unsigned)na;
   cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
   return e == cudaSuccess ? cudaGetLastError() : e;
-}
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              int cluster, Args... args) {
-  return launch_ex(kernel, grid, block, smem, stream, cluster, pdl_enabled(), args...);
 }
 #endif
 
@@ -90,19 +80,19 @@ constexpr int kConvMaxAcc = 8;
 constexpr int kConvThreads = 352;     // two groups
 constexpr int kConvMaxThreads = 480;  // three groups
 inline int conv_threads_for(int egroups) { return (7 + 4 * (egroups - 1)) * 32; }
-// groups for a 1-CTA-per-SM launch: at most one per accumulator stage (a group may only wait one phase ahead)
+// groups for a 1-CTA-per-SM launch: three, but at most one per accumulator stage (a group may only wait one phase ahead)
 inline int conv_pick_egroups(int acc_stages) {
-  const char* e = getenv("PADEL_B200_CONV_EGROUPS");
-  int want = e ? atoi(e) : 3;
-  if (want < 1 || want > 3) want = 3;
-  if (want > acc_stages) want = acc_stages;
+  const int want = acc_stages < 3 ? acc_stages : 3;
   return want < 1 ? 1 : want;
 }
-// PADEL_B200_CONV_OCC2: 0 = never two CTAs per SM, 1 = light many-tile layers, 2 (default) = also tiny layers
-inline int conv_occ_mode() {
-  const char* e = getenv("PADEL_B200_CONV_OCC2");
-  const int m = e ? atoi(e) : 1;
-  return m < 0 || m > 2 ? 1 : m;
+// Test / bring-up overrides of the kernel choice, never set by the product: tests/test_conv_gpu.py uses them to run the
+// per-tap and the halo kernel, and the CTA-pair mode, on the same shapes.  Read at every plan build.
+//   PADEL_B200_CONV_HALO: 0 = per-tap kernel only, 1 = halo kernel wherever it applies
+//   PADEL_B200_CONV_PAIR: 0 = no CTA pairs, 1 = CTA pairs wherever they apply
+// Returns the variable's value, or 2 when it is unset: the product rule.
+inline int conv_override(const char* name) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : 2;
 }
 constexpr int kConvMaxCout = 2048;  // ResNet50 layer4 (keypoints_tracker.py:158)
 
@@ -151,7 +141,7 @@ struct ConvKParams {
   int acc_stages, acc_cols;  // TMEM accumulator ring: acc_stages buffers, acc_cols columns apart
   int tmem_cols;             // TMEM columns allocated by the CTA (power of two; 512 unless two CTAs share an SM)
   int pair;                  // 1: CTA-pair mode (cluster of 2, cta_group::2 UMMAs issued by the even CTA)
-  int egroups;               // epilogue warp groups (1 with 224 threads / two CTAs per SM, else 2 or 4)
+  int egroups;               // epilogue warp groups (1 with 224 threads / two CTAs per SM, else 2 or 3)
   const float* head_w;
   const float* head_b;
   int head_n;
@@ -163,7 +153,6 @@ struct ConvKParams {
   int hs_ntaps, hs_sbo_rows, hs_x0, hs_y0, hs_tile_h;  // taps served from the halo, 8-row group stride (rows), box origin offsets
   int hs_tap_off[9];                                   // smem row offset of each tap's first pixel
   int hs_tap_desc[9];                                  // the same in 16-byte descriptor units (offset * row_bytes / 16)
-  int dbg_flags;   // PADEL_B200_CONV_DEBUG: bit0 = plain two-MUFU SiLU (default: one reciprocal per four values), bit1 = no fast epilogue
   long long* dbg;  // optional timeline buffer (CTA 0, first 64 tiles): [role 0..2][64][4] clock64 stamps
 };
 
@@ -176,7 +165,6 @@ struct ConvPlan {
   int threads;
   size_t smem_bytes;
   int variant;  // 0 = per-tap boxes (conv_tc_kernel), 1 = shared halo tile (conv_halo_kernel)
-  int pdl;      // programmatic dependent launch for this plan (captured from pb_set_plan_options at build time)
   int epi;      // PB_EPI_*: which epilogue instantiation of the kernel this layer runs
 };
 
@@ -191,6 +179,14 @@ int conv_epi_class(const pb_conv_desc* d, const ConvKParams& kp);
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+// Tensor maps shared by the conv set-ups (conv_halo.cu); both return 0, or 1 with the error set.
+// K-major weights [taps][cout_pad][cin], box (box_k x box_n x box_taps), swizzled to the box_k * 2-byte rows:
+int conv_weight_tmap(CUtensorMap* map, EncodeTiledFn encode, const pb_conv_desc* d, int taps, int box_k, int box_n,
+                     int box_taps);
+// NHWC activations as the 5-D view (s*C, W/s, s, H/s, N) -- for stride 2 a row holds a horizontal pixel pair and dim 2
+// is the image-row parity -- box (box_c, box_w, box_s, box_h, box_n), swizzled to the box_c * 2-byte rows:
+int conv_act_tmap(CUtensorMap* map, EncodeTiledFn encode, const pb_conv_desc* d, int s, int box_c, int box_w,
+                  int box_s, int box_h, int box_n);
 int conv_halo_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode);  // -1: not applicable
 int conv_stem_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode);
 int conv_halo_s2_setup(const pb_conv_desc* d, ConvPlan* plan, EncodeTiledFn encode);  // -1: not applicable
@@ -203,10 +199,6 @@ int conv_reference_launch(const pb_conv_desc* d, cudaStream_t stream);
 // aux kernels (aux_kernels.cu)
 int launch_maxpool2(const void* in, int N, int H, int W, int C, int c_off, int c, void* out, int out_C,
                     int out_coff, cudaStream_t s);
-int launch_upsample2(const void* in, int N, int H, int W, int C, int c_off, int c, void* out, int out_C,
-                     int out_coff, cudaStream_t s);
 int launch_sppf_pool(void* buf, int N, int H, int W, int C, int c, cudaStream_t s);
-int launch_pointwise_head(const void* in, int N, int H, int W, int C, const float* w, const float* b, int n_out,
-                          float* out, cudaStream_t s);
 
 }  // namespace pb

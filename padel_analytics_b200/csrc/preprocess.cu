@@ -346,17 +346,13 @@ int pb_pil_resize_u8(const uint8_t* src, int B, int Hs, int Ws, uint8_t* tmp, ui
   PB_CHECK(f16_layout >= 0 && f16_layout <= 2, "pil_resize: bad f16_layout");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const size_t hsmem = (((size_t)Ws * 3 + 15) & ~(size_t)15) + (size_t)Ws * 4;
-  // R rows per CTA when the source rows are whole 48-byte groups (every video format in practice); PADEL_B200_PIL_ROWS=1
-  // selects the one-row kernel (A/B)
-  static const int rows_env = [] {
-    const char* e = getenv("PADEL_B200_PIL_ROWS");
-    return e ? atoi(e) : 4;
-  }();
+  // 4 (or 2) rows per CTA when the source rows are whole 48-byte groups (every video format in practice) and 16-byte
+  // aligned; one row per CTA otherwise
   const long rows_total = (long)B * Hs;
   const size_t smem4 = (size_t)4 * Ws * 4 + (size_t)4 * Wo * 3;
   const size_t smem2 = (size_t)2 * Ws * 4 + (size_t)2 * Wo * 3;
-  if (rows_env >= 2 && Ws % 16 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0 && smem2 <= 200 * 1024) {
-    if (rows_env >= 4 && smem4 <= 100 * 1024) {
+  if (Ws % 16 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0 && smem2 <= 200 * 1024) {
+    if (smem4 <= 100 * 1024) {
       PB_CUDA((cudaError_t)ensure_dynamic_smem(reinterpret_cast<const void*>(&pil_horizontal_rows_kernel<4>), smem4));
       pil_horizontal_rows_kernel<4><<<(unsigned)((rows_total + 3) / 4), 256, smem4, s>>>(src, Ws, rows_total, tmp, Wo,
                                                                                          bounds_h, kk_h, ksize_h, swap_rb);

@@ -128,7 +128,7 @@ class Program:
         self._h = L.lib().pb_program_create()
         self._keep = []  # tensors referenced by raw pointer
         self.descs: list = []  # per op: ConvDesc copy (convs) or None
-        self.kinds: list[str] = []  # per op: 'conv' | 'pool' | 'up' | 'sppf'
+        self.kinds: list[str] = []  # per op: 'conv' | 'pool' | 'sppf'
         self.flops: list[float] = []  # per op: algorithmic FLOPs (2*MACs on the real, unpadded channel counts)
         self.bytes: list[float] = []  # per op: algorithmic activation bytes (input read once + output written once)
 
@@ -159,25 +159,10 @@ class Program:
                                                 out.shape[-1], out_coff))
         self._note("pool", N * H * W * c * 2 * 1.25)
 
-    def upsample2(self, x, c_off, c, out, out_coff):
-        N, H, W, Ct = x.shape
-        L.check(L.lib().pb_program_add_upsample2(self._h, x.data_ptr(), N, H, W, Ct, c_off, c, out.data_ptr(),
-                                                 out.shape[-1], out_coff))
-        self._note("up", N * H * W * c * 2 * 5.0)
-
     def sppf_pool(self, buf, c):
         N, H, W, Ct = buf.shape
         L.check(L.lib().pb_program_add_sppf_pool(self._h, buf.data_ptr(), N, H, W, Ct, c))
         self._note("sppf", N * H * W * c * 2 * 4.0)
-
-    def pointwise_head(self, x, weight, bias, out):
-        N, H, W, Ct = x.shape
-        L.check(L.lib().pb_program_add_pointwise_head(self._h, x.data_ptr(), N, H, W, Ct, weight.data_ptr(),
-                                                      bias.data_ptr(), weight.shape[0], out.data_ptr()))
-        self.kinds.append("head")
-        self.descs.append(None)
-        self.flops.append(2.0 * N * H * W * Ct * weight.shape[0])
-        self.bytes.append(float(N * H * W * (Ct * 2 + weight.shape[0] * 4)))
 
     def _note(self, kind: str, nbytes: float):
         self.kinds.append(kind)
@@ -190,8 +175,7 @@ class Program:
         return L.lib().pb_program_num_ops(self._h)
 
     def op_kernels(self) -> list[str]:
-        names = {0: "conv_tc_kernel", 1: "conv_halo_kernel", 2: "maxpool2_kernel", 3: "upsample2_kernel",
-                 4: "sppf_pool_kernel", 5: "pointwise_head_kernel"}
+        names = {0: "conv_tc_kernel", 1: "conv_halo_kernel", 2: "maxpool2_kernel", 4: "sppf_pool_kernel"}
         return [names[L.lib().pb_program_op_kernel(self._h, i)] for i in range(self.num_ops)]
 
     def run(self, first: int | None = None, last: int | None = None):

@@ -8,8 +8,6 @@ Network definition being replaced: /root/reference/trackers/ball_tracker/models.
 """
 from __future__ import annotations
 
-import os
-
 import numpy as np
 import torch
 
@@ -61,12 +59,9 @@ class TrackNetEngine:
                                    sd[f"{p}.bn.bias"].float(), sd[f"{p}.bn.running_mean"].float(),
                                    sd[f"{p}.bn.running_var"].float(), 1e-5)
                 self._w[p] = ops.pack_conv_weight(w, b, ops.pad16(ci) if ci != 27 else 32, cout, self.device)
-        # predictor 1x1 (64 -> 8) + sigmoid.  Default: a 1x1 tensor-core conv (fp16 weights, N = 16) writing the fp32
-        # NCHW planes -- HBM-bound at ~4.8 TB/s, 158 us per 32 frames.  PADEL_B200_TRACKNET_HEAD=pointwise selects the
-        # CUDA-core kernel with fp32 weights instead (308 us: ~800 instructions per 32 pixels, issue-bound).  The
-        # fused-epilogue variant of the conv kernel also exists but costs more (512 FMAs per pixel in the epilogue).
-        self._head_w = sd["predictor.weight"].float().reshape(8, 64).contiguous().to(self.device)
-        self._head_b = sd["predictor.bias"].float().contiguous().to(self.device)
+        # predictor 1x1 (64 -> 8) + sigmoid: a 1x1 tensor-core conv (fp16 weights, N = 16) writing the fp32 NCHW planes
+        # -- HBM-bound at ~4.8 TB/s, 158 us per 32 frames (a CUDA-core kernel with fp32 weights took 308 us, issue-bound).
+        # The fused-epilogue variant of the conv kernel also exists but costs more (512 FMAs per pixel in the epilogue).
         self._w["predictor"] = ops.pack_conv_weight(sd["predictor.weight"].float().reshape(8, 64, 1, 1),
                                                     sd["predictor.bias"].float(), 64, 16, self.device)
         self._build()
@@ -94,18 +89,6 @@ class TrackNetEngine:
         self.pred = torch.zeros((7 + B, 8, H, W), dtype=torch.float32, device=dev)
 
     def _build(self):
-        # PADEL_B200_BALL_SMS=n: size this program's persistent grids for n SMs (and launch its kernels without
-        # programmatic overlap, so a waiting successor never parks on the SMs left free) -- for running beside the YOLO
-        # chains of the other trackers (FusedPass streams mode 2) instead of before / after them
-        sms = int(os.environ.get("PADEL_B200_BALL_SMS", "0"))
-        if sms > 0:
-            L.lib().pb_set_plan_options(sms, 0)
-        try:
-            self._build_program()
-        finally:
-            L.lib().pb_set_plan_options(0, -1)
-
-    def _build_program(self):
         P = ops.Program()
         W_ = self._w
         R, UP, SIG = L.ACT_RELU, L.OUT_F16_NHWC_UP2, L.ACT_SIGMOID
@@ -117,17 +100,12 @@ class TrackNetEngine:
                    cin_real=27 if name == "down_block_1.conv_1" else cin)
 
         # MaxPool2d of the first two encoder blocks (models.py:60,62) is a second store of the producing conv
-        # (PB_OUT2_POOL2); PADEL_B200_FUSE_OUT2=0 keeps the separate pool launches (A/B)
-        fuse = os.environ.get("PADEL_B200_FUSE_OUT2", "1") != "0"
-
+        # (PB_OUT2_POOL2).  The third one stays a launch: its 256-channel conv runs on the per-tap kernel, which has no
+        # pooled store.
         conv(self.x, 0, 32, "down_block_1.conv_1", self.t1, 0)
-        conv(self.t1, 0, 64, "down_block_1.conv_2", self.cat3, 128, pool=self.p1 if fuse else None)
-        if not fuse:
-            P.maxpool2(self.cat3, 128, 64, self.p1, 0)
+        conv(self.t1, 0, 64, "down_block_1.conv_2", self.cat3, 128, pool=self.p1)
         conv(self.p1, 0, 64, "down_block_2.conv_1", self.t2, 0)
-        conv(self.t2, 0, 128, "down_block_2.conv_2", self.cat2, 256, pool=self.p2 if fuse else None)
-        if not fuse:
-            P.maxpool2(self.cat2, 256, 128, self.p2, 0)
+        conv(self.t2, 0, 128, "down_block_2.conv_2", self.cat2, 256, pool=self.p2)
         conv(self.p2, 0, 128, "down_block_3.conv_1", self.t3a, 0)
         conv(self.t3a, 0, 256, "down_block_3.conv_2", self.t3b, 0)
         conv(self.t3b, 0, 256, "down_block_3.conv_3", self.cat1, 512)
@@ -143,10 +121,7 @@ class TrackNetEngine:
         conv(self.cat3, 0, 192, "up_block_3.conv_1", self.u3a, 0)
         self._pred_new = self.pred[7:]
         conv(self.u3a, 0, 64, "up_block_3.conv_2", self.u3b, 0)
-        if os.environ.get("PADEL_B200_TRACKNET_HEAD", "tc") == "tc":
-            conv(self.u3b, 0, 64, "predictor", self._pred_new, 0, L.OUT_F32_NCHW, SIG, k=1, store=8)
-        else:
-            P.pointwise_head(self.u3b, self._head_w, self._head_b, self._pred_new)
+        conv(self.u3b, 0, 64, "predictor", self._pred_new, 0, L.OUT_F32_NCHW, SIG, k=1, store=8)
         self.prog = P
 
     # -- execution ---------------------------------------------------------------------------------------------

@@ -10,7 +10,6 @@ reads and writes (no copies except the two nearest-upsamples and SPPF pooling).
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass
 
 import numpy as np
@@ -229,8 +228,7 @@ class YoloEngine:
             conv(cat, 0, ccat, f"{pre}.cv2", out, ooff, 1, 1, up=up)
 
         # the two nn.Upsample(2, "nearest") of the neck (layers 10, 13) are a second, replicated store of the
-        # producing 1x1 conv (PB_OUT2_UP2); PADEL_B200_FUSE_OUT2=0 keeps the separate upsample launches (A/B)
-        fuse = os.environ.get("PADEL_B200_FUSE_OUT2", "1") != "0"
+        # producing 1x1 conv (PB_OUT2_UP2)
         c0, c1, c2, c3, c4 = (self._cout(f"model.{i}") for i in (0, 1, 3, 5, 7))
         for c in (c0, c1, c2, c3, c4):
             if c % 16:
@@ -266,12 +264,8 @@ class YoloEngine:
         c2f(b7, 0, c4, 8, b8, 0, True)
         conv(b8, 0, c4, "model.9.cv1", sp, 0, 1, 1)  # SPPF
         P.sppf_pool(sp, c4 // 2)
-        conv(sp, 0, 4 * (c4 // 2), "model.9.cv2", cat20, c3, 1, 1, up=cat11 if fuse else None)  # P5 (+ layers 10-11)
-        if not fuse:
-            P.upsample2(cat20, c3, c4, cat11, 0)  # layers 10-11
-        c2f(cat11, 0, c4 + c3, 12, cat17, c2, False, up=cat14 if fuse else None)  # h4 (+ layers 13-14)
-        if not fuse:
-            P.upsample2(cat17, c2, c3, cat14, 0)  # layers 13-14
+        conv(sp, 0, 4 * (c4 // 2), "model.9.cv2", cat20, c3, 1, 1, up=cat11)  # P5 (+ layers 10-11)
+        c2f(cat11, 0, c4 + c3, 12, cat17, c2, False, up=cat14)  # h4 (+ layers 13-14)
         c2f(cat14, 0, c3 + c2, 15, o3, 0, False)
         conv(o3, 0, c2, "model.16", cat17, 0, 3, 2)
         c2f(cat17, 0, c2 + c3, 18, o4, 0, False)

@@ -1,7 +1,6 @@
 """Whole-program device time of the four conv programs (CUDA events around `reps` back-to-back runs, no per-op
 events in between, so programmatic dependent launch can overlap consecutive kernels).
-Usage: python scripts/prog_times.py [B] [reps]   (compare PADEL_B200_PDL=0 / 1 in separate processes)"""
-import os
+Usage: python scripts/prog_times.py [B] [reps]"""
 import sys
 
 import torch
@@ -22,7 +21,7 @@ for k in ("players", "pose", "court"):
 progs = {"ball": tr["ball"].tracknet.prog}
 for k in ("players", "pose", "court"):
     progs[k] = list(tr[k].model._progs.values())[0]["prog"]
-print("PDL", os.environ.get("PADEL_B200_PDL", "1"), "B", B)
+print("B", B)
 for name, p in progs.items():
     for _ in range(3):
         p.run()
